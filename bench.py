@@ -100,7 +100,15 @@ def parse():
     ap.add_argument("--syncbn", action="store_true",
                     help="BatchNorm statistics all-reduced over the ranks (equals single-process "
                          "training on the global batch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one computed (loss, "
+                         "predictions, parameters, gradients, BatchNorm statistics of rank 0) as "
+                         "DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm only")
     metric, batch, conv, mode, shape, tuples = WORKLOADS[args.workload]
     args.metric, args.mode, args.shape, args.tuples = metric, mode, shape, tuples
     args.batch = args.batch or batch
@@ -222,6 +230,30 @@ def host_batches(args, per_gpu, rank, count, world=1):
                 mine.append(g)
         out.append(collate([graphs[g] for g in sorted(mine)]))
     return out
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Write every named array as ``out_dir/<name>.npy`` in float32 (float64 stays float64).
+    When the files would exceed `budget` bytes together, every array keeps the same fraction of
+    its elements: a sample of flat positions drawn with a fixed seed and kept in ascending order,
+    so two runs with the same arguments write the same positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: a if a.dtype == np.float64 else a.astype(np.float32, copy=False)
+              for k, a in arrays.items()}
+    header = 256                                   # upper bound of one .npy header here
+    data = sum(a.nbytes for a in arrays.values())
+    room = budget - header * len(arrays)
+    frac = 1.0 if data <= room else room / data
+    for name, a in arrays.items():
+        if frac < 1.0:
+            keep = int(a.size * frac)
+            pos = np.random.default_rng(0).choice(a.size, keep, replace=False)
+            a = a.reshape(-1)[np.sort(pos)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def batch_stats(args, hb, keys):
@@ -584,7 +616,8 @@ def run_b200(args):
             pin_host_batch(hb, pinned)
     h2d_bytes = int(np.mean([hb.nbytes() for hb in hbs]))
 
-    def train_step(dd):
+    def step_outputs(dd):
+        """(loss, predictions) of one optimisation step on `dd`."""
         bucket.zero()
         pred, y = model(dd), dd["y"].unsqueeze(-1)
         nv = dd.get("num_valid_graphs")           # capacity-padded batch: drop the dummy graph
@@ -597,7 +630,10 @@ def run_b200(args):
             opt.step()
         else:
             opt.step(1.0 / bucket.allreduce_sum())
-        return loss
+        return loss, pred.detach()
+
+    def train_step(dd):
+        return step_outputs(dd)[0]
 
     def barrier():
         if world > 1:
@@ -610,7 +646,7 @@ def run_b200(args):
         l0 = _lib.launches()
         e0.record()
         for i in range(steps):
-            fn(i)
+            last = fn(i)
             if per_step is not None:
                 ev = torch.cuda.Event(enable_timing=True)
                 ev.record()
@@ -625,7 +661,7 @@ def run_b200(args):
         if per_step is not None:
             evs = [e0] + per_step
             per_step[:] = [a.elapsed_time(b) for a, b in zip(evs[:-1], evs[1:])]
-        return float(ms.item()), _lib.launches() - l0
+        return float(ms.item()), _lib.launches() - l0, last
 
     warm = max(3, args.warmup)
     for i in range(warm):
@@ -637,7 +673,7 @@ def run_b200(args):
     if not args.no_graph:
         try:
             from pygho_b200.graph import StepGraph
-            graphs = [StepGraph(lambda dd=dd: train_step(dd), warmup=1) for dd in dds]
+            graphs = [StepGraph(lambda dd=dd: step_outputs(dd), warmup=1) for dd in dds]
             graph_note = f"cuda graph replay, one graph per resident batch ({len(graphs)})"
         except Exception as e:  # noqa: BLE001
             graphs = None
@@ -647,15 +683,22 @@ def run_b200(args):
     if graphs is not None:
         run_step = lambda i: graphs[i % len(graphs)].replay()  # noqa: E731
     else:
-        run_step = lambda i: train_step(dds[i % len(dds)])  # noqa: E731
+        run_step = lambda i: step_outputs(dds[i % len(dds)])  # noqa: E731
     for i in range(warm):
         run_step(i)
     # clocks / throttle reasons are sampled by rank 0 only (its own GPU): eight nvidia-smi pollers
     # contend for the driver lock and slow the graph launches of every rank
     with ClockSampler(local if rank == 0 else -1) as clocks:
-        ms_total, launches = timed(run_step, args.steps)
+        ms_total, launches, (last_loss, last_pred) = timed(run_step, args.steps)
     if graphs is not None:                                # replays do not pass through Python
         launches = sum(graphs[i % len(graphs)].launches for i in range(args.steps))
+    if args.dump_outputs and rank == 0:
+        named = dict(model.named_parameters())
+        arrays = {"loss": last_loss.reshape(1), "pred": last_pred}
+        arrays.update({f"param.{k}": p for k, p in named.items()})
+        arrays.update({f"grad.{k}": p.grad for k, p in named.items() if p.grad is not None})
+        arrays.update({f"buffer.{k}": b for k, b in model.named_buffers() if b.is_floating_point()})
+        dump_outputs(args.dump_outputs, {k: v.detach().cpu().numpy() for k, v in arrays.items()})
     clock_summary = clocks.summary()
     ms_step = ms_total / args.steps
     value = glob / (ms_step * 1e-3)
@@ -739,7 +782,7 @@ def run_b200(args):
         gc.collect()
         gc.freeze()    # long-lived objects out of the collector's way: no multi-ms gen-2 pauses
         per_step = []
-        e2e_ms, _ = timed(e2e_step, args.steps, finish=read_pending, per_step=per_step)
+        e2e_ms, _, _ = timed(e2e_step, args.steps, finish=read_pending, per_step=per_step)
         assert len(losses) == args.steps and all(np.isfinite(losses)), "e2e: every step's loss is read"
         if os.environ.get("PYGHO_B200_BENCH_TRACE"):
             print(f"[trace] rank {rank} e2e device ms per step: {[round(v, 2) for v in per_step]}",

@@ -47,6 +47,39 @@ def test_own_arm_needs_a_gpu():
     assert "no CPU path" in (r.stderr + r.stdout)
 
 
+def test_steps_below_one_are_refused():
+    r = run(["--impl", "reference", "--steps", "0"])
+    assert r.returncode != 0 and "--steps must be at least 1" in r.stderr
+
+
+def test_dump_outputs_writes_float_arrays_within_the_budget(tmp_path):
+    """--dump-outputs: every array as <name>.npy in float32 (float64 kept); above the byte budget
+    the same seeded sample of positions in every run."""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    rng = np.random.default_rng(1)
+    arrays = {"loss": np.float32([0.5]), "pred": rng.standard_normal((50, 1)).astype(np.float32),
+              "param.w": rng.standard_normal((300, 200)), "count": np.arange(7)}
+    b.dump_outputs(str(tmp_path / "all"), arrays)
+    for k, v in arrays.items():
+        got = np.load(tmp_path / "all" / f"{k}.npy")
+        assert got.dtype == (np.float64 if v.dtype == np.float64 else np.float32), k
+        assert np.array_equal(got, v), k
+    budget = 100_000
+    for d in ("a", "b"):
+        b.dump_outputs(str(tmp_path / d), arrays, budget=budget)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(f"{k}.npy" for k in arrays)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= budget
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)), f
+    w = np.load(tmp_path / "a" / "param.w.npy")
+    assert 0 < w.size < arrays["param.w"].size and np.isin(w, arrays["param.w"]).all()
+
+
 def test_reference_arm_other_workloads():
     """The dense PPGN and the sr25 DSSGNN / I2 arms run on the CPU oracle too."""
     for wl in ("ppgn_dd", "dssgnn_sr25", "i2_sr25"):

@@ -97,9 +97,10 @@ def test_host_generator_matches_oracle_sampler():
 
 def test_sr25_like_graphs_are_strongly_regular():
     """The synthetic cfg4 graphs have the sr25 parameters (25, 12, 5, 6) and the tuple / triple
-    counts SURVEY.md section 8 quotes for sr25; where the reference's dataset is mounted they are
-    isomorphic to members of dataset/sr25/raw/sr251256.g6."""
-    import os
+    counts SURVEY.md section 8 quotes for sr25.  The reference's sr25 dataset holds all 15
+    strongly regular graphs with these parameters (Paulus), so the two Latin-square graphs are
+    members of it, and distinct ones because they are not isomorphic."""
+    import networkx as nx
     from pygho_b200.hodata.synthetic import make_batch, sr25_like_graph
     rng = np.random.default_rng(0)
     mats = []
@@ -115,10 +116,4 @@ def test_sr25_like_graphs_are_strongly_regular():
         mats.append(A)
     hb = make_batch(2, seed=1, tuples="i2", shape="sr25")
     assert hb.tupleid.shape == (3, 2 * 7500) and hb.tuplefeat.shape == (2 * 7500, 2)
-    path = "/root/reference/dataset/sr25/raw/sr251256.g6"
-    if os.path.exists(path):
-        import networkx as nx
-        ref = nx.read_graph6(path)
-        hits = [[i for i, H in enumerate(ref) if nx.is_isomorphic(nx.from_numpy_array(A), H)]
-                for A in mats]
-        assert all(len(h) == 1 for h in hits) and hits[0] != hits[1]
+    assert not nx.is_isomorphic(nx.from_numpy_array(mats[0]), nx.from_numpy_array(mats[1]))
