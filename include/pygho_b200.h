@@ -39,10 +39,12 @@ const char* pgh_last_error(void);
 int pgh_abi_version(void);
 /* fills {device ordinal, SM count, L2 bytes, cc major, cc minor}; host pointer */
 int pgh_device_info(int32_t* out5);
-/* run-time tuning knobs (only the work split changes; reductions stay deterministic for a
- * given setting): key 0 = seg_gmr kernel variant (-1 built-in choice), key 1 = ring kernel
- * plan entries per warp, keys 2..5 = fused BatchNorm kernels (CTAs per SM, rows in flight,
- * reverse walk, forward elements in flight; 0 = default); host call */
+/* run-time tuning knobs; host call.  Keys 2..5 = fused BatchNorm kernels (CTAs per SM, rows in
+ * flight, reverse walk, forward elements in flight; 0 = default): only the work split changes,
+ * reductions stay deterministic for a given setting.  Key 7 = bit mask of mamamm profiling
+ * ablations (0 = off, the default; others switch parts of the kernel off).  Key 8 = programmatic dependent
+ * launch (1 = on, the default; 0 = every kernel fully serialised).  Any other key is an
+ * argument error. */
 int pgh_set_tuning(int key, int value);
 /* profiling hook: device buffer of n_words uint64 that the pipelined mamamm kernel fills
  * with %globaltimer stamps of its three warp roles (CTA 0 only); NULL switches it off */
@@ -73,21 +75,6 @@ int pgh_seg_gmr_ld_f32(const float* a_val, int64_t lda, const int32_t* c, const 
                        const float* b_val, int64_t ldb, const int32_t* d, const int32_t* rowptr,
                        int64_t n_rows, int64_t n_entries, int64_t dense, int aggr, int accumulate,
                        float* out, int64_t ldo, void* stream);
-
-/* Shared-memory staging of a tile's first-operand row range (dense == 128, two operands, sum or
- * mean; BASELINE north_star "staging of each row's key range").  pgh_tile_ranges finds, for every
- * tile of `rows_per_tile` consecutive output rows, the range [lo, lo + cnt) of first-operand rows
- * its plan entries reference (once per batch, cached with the plan); pgh_seg_gmr_staged_f32 copies
- * that range to shared memory once per tile when cnt <= max_stage_rows (<= 256) and reduces the
- * tile's rows from it -- same arguments, reduction order and results as pgh_seg_gmr_ld_f32. */
-int pgh_tile_ranges(const int32_t* rowptr, const int32_t* first, int64_t n_rows,
-                    int64_t rows_per_tile, int32_t* tile_lo, int32_t* tile_cnt, void* stream);
-int pgh_seg_gmr_staged_f32(const float* a_val, int64_t lda, const int32_t* c, const float* a_scale,
-                           const float* b_val, int64_t ldb, const int32_t* d,
-                           const int32_t* rowptr, int64_t n_rows, int64_t dense, int aggr,
-                           int accumulate, const int32_t* tile_lo, const int32_t* tile_cnt,
-                           int64_t rows_per_tile, int64_t max_stage_rows, float* out, int64_t ldo,
-                           void* stream);
 
 /* pgh_seg_gmr_ld_f32 with a fused row epilogue (dense % 128 == 0, 16-byte aligned rows, sum or
  * mean):  out[r,:] = add_src[r,:] + reduction(r) (+ add_src2[r,:])   and, if copy_src != NULL,

@@ -29,9 +29,6 @@ SIGNATURES = {
     "pgh_seg_gmr_ld_f32": (_i, [_p, _i64, _p, _p, _p, _i64, _p, _p, _i64, _i64, _i64, _i, _i, _p, _i64, _p]),
     "pgh_seg_gmr_fused_f32": (_i, [_p, _i64, _p, _p, _p, _i64, _p, _p, _i64, _i64, _i64, _i, _p, _i64,
                                    _p, _i64, _p, _i64, _p, _i64, _p, _i64, _p]),
-    "pgh_tile_ranges": (_i, [_p, _p, _i64, _i64, _p, _p, _p]),
-    "pgh_seg_gmr_staged_f32": (_i, [_p, _i64, _p, _p, _p, _i64, _p, _p, _i64, _i64, _i, _i, _p, _p, _i64,
-                                    _i64, _p, _i64, _p]),
     "pgh_seg_tie_scale_f32": (_i, [_p, _p, _p, _p, _p, _i64, _i64, _p, _p, _p, _p]),
     "pgh_seg_select_bwd_f32": (_i, [_p, _p, _p, _p, _p, _i64, _i64, _p, _p, _p, _p]),
     "pgh_inv_count_f32": (_i, [_p, _i64, _p, _p]),

@@ -13,7 +13,6 @@
 // 4*dense*(nA + nB + n_rows) + 4*(2T + n_rows + 1)  (SURVEY.md section 8d).
 #include <math.h>
 #include <stdarg.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -162,126 +161,21 @@ seg_gmr_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
   }
 }
 
-// Streaming variant for dense % 128 == 0 (the benchmark width): a warp owns kRW consecutive
-// output rows and walks ALL their plan entries as one stream, kSU entries (2*kSU row loads of
-// 512 B) in flight per lane regardless of row boundaries.  The ZINC-shaped plans have ~2
-// entries per row, so batching loads across rows is what turns a latency-bound kernel
-// (rowptr -> plan -> values chain per row) into a bandwidth-bound one.  Row boundaries are
-// warp-uniform (every lane handles the same entry, lanes = columns), so the flush of a
-// finished row is a plain uniform branch and one coalesced 512 B store.
-constexpr int kMaxRW = 16;  // rows per warp upper bound (<= 31: lane i holds rowptr[r0 + i])
-// plan entries in flight per lane: 4 with two operands (8 x 128-bit loads), 8 with one
-
-template <int AGGR, bool HAS_B, int kSU, int MINB>
-__global__ void __launch_bounds__(kThreads, MINB)
-seg_gmr_stream_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
-                      const float* __restrict__ a_scale, const float* __restrict__ b_val,
-                      const int* __restrict__ d, const int* __restrict__ rowptr,
-                      long long n_rows, int dense, int lda, int ldb, int ldo, int rw, int accum,
-                      float* __restrict__ out) {
-  pdl_enter();
-  constexpr unsigned kFull = 0xffffffffu;
-  const int lane = threadIdx.x & 31;
-  const long long warp = (long long)blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5);
-  const long long r0 = warp * rw;
-  if (r0 >= n_rows) return;
-  const int nr = (int)min((long long)rw, n_rows - r0);
-  int rp = 0;
-  if (lane <= nr) rp = rowptr ? __ldg(rowptr + r0 + lane) : (int)(r0 + lane);
-  const int e_beg = __shfl_sync(kFull, rp, 0);
-  const int e_end = __shfl_sync(kFull, rp, nr);
-  const float init = (AGGR == PGH_MAX) ? -INFINITY : (AGGR == PGH_MIN) ? INFINITY : 0.f;
-  for (int col = lane * 4; col < dense; col += 128) {
-    const float* __restrict__ a_col = a_val + col;
-    const float* __restrict__ b_col = HAS_B ? b_val + col : nullptr;
-    float* __restrict__ o_col = out + (size_t)r0 * ldo + col;
-    float4 acc = make_float4(init, init, init, init);
-    int cur = 0;                                    // local index of the row being reduced
-    int cur_beg = e_beg;
-    int cur_end = __shfl_sync(kFull, rp, 1);
-// finish the current row: one coalesced 512 B store, then advance (warp-uniform)
-#define PGH_FLUSH()                                                                     \
-  do {                                                                                  \
-    const int len_ = cur_end - cur_beg;                                                 \
-    float4 r_ = acc;                                                                    \
-    if (len_ == 0) r_ = make_float4(0.f, 0.f, 0.f, 0.f);                                \
-    else if (AGGR == PGH_MEAN) {                                                        \
-      const float n_ = (float)len_;                                                     \
-      r_ = make_float4(acc.x / n_, acc.y / n_, acc.z / n_, acc.w / n_);                 \
-    }                                                                                   \
-    if (accum == 1) {                                                                   \
-      const float4 o_ = *reinterpret_cast<const float4*>(o_col + (size_t)cur * ldo);    \
-      r_ = make_float4(__fadd_rn(o_.x, r_.x), __fadd_rn(o_.y, r_.y),                    \
-                       __fadd_rn(o_.z, r_.z), __fadd_rn(o_.w, r_.w));                   \
-    }                                                                                   \
-    /* accum == 2: profiling mode (tuning key 6), the row store is skipped */           \
-    if (accum != 2 || r_.x == 1.2345e-30f)                                              \
-      *reinterpret_cast<float4*>(o_col + (size_t)cur * ldo) = r_;                       \
-    acc = make_float4(init, init, init, init);                                          \
-    ++cur;                                                                              \
-    cur_beg = cur_end;                                                                  \
-    cur_end = __shfl_sync(kFull, rp, min(cur + 1, 31));                                 \
-  } while (0)
-    for (int base = e_beg; base < e_end; base += 32) {
-      const int t = base + lane;
-      int ci = 0, di = 0;
-      float sc = 1.f;
-      if (t < e_end) {
-        ci = c ? __ldg(c + t) : t;
-        if (HAS_B) di = d ? __ldg(d + t) : t;
-        if (a_scale) sc = __ldg(a_scale + ci);
-      }
-      const int chunk = min(32, e_end - base);
-#pragma unroll 1
-      for (int k = 0; k < chunk; k += kSU) {
-        float4 av[kSU], bv[kSU];
-        float ss[kSU];
-        // all 2*kSU loads are unconditional (indices clamped to the last valid entry) so
-        // that they are issued back to back and stay in flight together
-#pragma unroll
-        for (int u = 0; u < kSU; ++u) {
-          const int kk = min(k + u, chunk - 1);
-          const int cc = __shfl_sync(kFull, ci, kk);
-          ss[u] = __shfl_sync(kFull, sc, kk);
-          av[u] = __ldg(reinterpret_cast<const float4*>(a_col + (size_t)cc * lda));
-          if (HAS_B) {
-            const int dd = __shfl_sync(kFull, di, kk);
-            bv[u] = __ldg(reinterpret_cast<const float4*>(b_col + (size_t)dd * ldb));
-          }
-        }
-#pragma unroll
-        for (int u = 0; u < kSU; ++u) {
-          if (k + u < chunk) {
-            const int tt = base + k + u;
-            while (tt >= cur_end) PGH_FLUSH();      // finished (or empty) rows
-            float4 m = make_float4(__fmul_rn(av[u].x, ss[u]), __fmul_rn(av[u].y, ss[u]),
-                                   __fmul_rn(av[u].z, ss[u]), __fmul_rn(av[u].w, ss[u]));
-            if (HAS_B)
-              m = make_float4(__fmul_rn(m.x, bv[u].x), __fmul_rn(m.y, bv[u].y),
-                              __fmul_rn(m.z, bv[u].z), __fmul_rn(m.w, bv[u].w));
-            if (AGGR == PGH_MAX)
-              acc = make_float4(fmaxf(acc.x, m.x), fmaxf(acc.y, m.y), fmaxf(acc.z, m.z), fmaxf(acc.w, m.w));
-            else if (AGGR == PGH_MIN)
-              acc = make_float4(fminf(acc.x, m.x), fminf(acc.y, m.y), fminf(acc.z, m.z), fminf(acc.w, m.w));
-            else
-              acc = make_float4(__fadd_rn(acc.x, m.x), __fadd_rn(acc.y, m.y),
-                                __fadd_rn(acc.z, m.z), __fadd_rn(acc.w, m.w));
-          }
-        }
-      }
-    }
-    while (cur < nr) PGH_FLUSH();
-#undef PGH_FLUSH
-  }
-}
-
-
 // ---------------------------------------------------------------------------------------
-// Lean streaming variant.  ncu on the kernel above (profiles/r1_seg_gmr_v3_issue.md): 32.2 M warp
-// instructions per launch = 69 per plan entry, i.e. 28.6 us of pure issue time on 148 SMs -- the
-// kernel is as much issue-bound as memory-bound (sm__throughput 49 %, DRAM 49 %).  Same work
-// split, same load batching and the same sequential reduction order, but everything the inner
-// loop does not need is compiled out or hoisted:
+// Lean streaming kernel for dense % 128 == 0 (the benchmark width): a warp owns rw consecutive
+// output rows and walks ALL their plan entries as one stream, U entries (2*U row loads of 512 B)
+// in flight per lane regardless of row boundaries.  The ZINC-shaped plans have ~2 entries per
+// row, so batching loads across rows is what turns a latency-bound kernel (rowptr -> plan ->
+// values chain per row) into a bandwidth-bound one.  Row boundaries are warp-uniform (every lane
+// handles the same entry, lanes = columns), so the flush of a finished row is a plain uniform
+// branch and one coalesced 512 B store.
+constexpr int kMaxRW = 16;  // rows per warp upper bound (<= 31: lane i holds rowptr[r0 + i])
+// ncu on the first streaming kernel of that design (profiles/r1_seg_gmr_v3_issue.md; archived in
+// profiles/probes/seg_gmr_retired_r2.cu.txt): 32.2 M warp instructions per launch = 69 per plan
+// entry, i.e. 28.6 us of pure issue time on 148 SMs -- it was as much issue-bound as memory-bound
+// (sm__throughput 49 %, DRAM 49 %).  This kernel keeps its work split, load batching and
+// sequential reduction order, but everything the inner loop does not need is compiled out or
+// hoisted:
 //   * a_scale / accumulate / mean are template parameters, not run-time tests per entry;
 //   * full groups of U entries run without index clamps or validity tests, the (single)
 //     partial group of a warp is a separate, guarded copy of the body;
@@ -446,14 +340,14 @@ seg_gmr_lean_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
 }
 
 // ---------------------------------------------------------------------------------------
-// Ring variant (dense % 128 == 0): same work split and the same sequential reduction order
-// as the streaming kernel, but the value rows travel global -> shared memory with cp.async
-// (LDGSTS, 16 B per lane = one 512 B row per warp instruction) into a per-lane FIFO of NS
-// stages, so the number of rows in flight is bounded by shared memory (NS x 1 KB per warp)
-// instead of registers.  A lane only ever reads back the 16 B it copied itself, so the
-// pipeline needs no barrier at all: cp.async.wait_group is per thread.  The plan of the
-// NEXT 32 entries is prefetched into registers while the current 32 are streamed, which
-// removes the plan-load bubble of the register-staged kernel.
+// Ring kernel (dense % 128 == 0, one operand: pooling, unpooling, coalesce): same work split
+// and the same sequential reduction order as the lean kernel, but the value rows travel
+// global -> shared memory with cp.async (LDGSTS, 16 B per lane = one 512 B row per warp
+// instruction) into a per-lane FIFO of NS stages, so the number of rows in flight is bounded by
+// shared memory (NS x 512 B per warp) instead of registers.  A lane only ever reads back the
+// 16 B it copied itself, so the pipeline needs no barrier at all: cp.async.wait_group is per
+// thread.  The plan of the NEXT 32 entries is prefetched into registers while the current 32
+// are streamed, which removes the plan-load bubble of the register-staged kernel.
 __device__ __forceinline__ void cp_async16(uint32_t saddr, const void* g) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 16;\n" ::"r"(saddr), "l"(g) : "memory");
 }
@@ -473,7 +367,8 @@ __device__ __forceinline__ float4 lds128(uint32_t saddr) {
   return v;
 }
 
-template <int AGGR, bool HAS_B, int NS, int U, int WARPS>
+// b_val, d and ldb are not read: the argument list is that of the row-wise kernel.
+template <int AGGR, int NS, int U, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32)
 seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
                     const float* __restrict__ a_scale, const float* __restrict__ b_val,
@@ -483,7 +378,6 @@ seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
   pdl_enter();
   static_assert(NS % U == 0 && 32 % U == 0 && NS <= 32, "ring geometry");
   constexpr unsigned kFull = 0xffffffffu;
-  constexpr int OPS = HAS_B ? 2 : 1;
   constexpr int NG = NS / U;                        // commit groups in flight
   extern __shared__ __align__(16) unsigned char ring_smem[];
   const int lane = threadIdx.x & 31;
@@ -496,13 +390,12 @@ seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
   if (lane <= nr) rp = rowptr ? __ldg(rowptr + r0 + lane) : (int)(r0 + lane);
   const int e_beg = __shfl_sync(kFull, rp, 0);
   const int e_end = __shfl_sync(kFull, rp, nr);
-  // stage s, operand o of this lane: ring + (s * OPS + o) * 512
+  // stage s of this lane: ring + s * 512
   const uint32_t ring = (uint32_t)__cvta_generic_to_shared(ring_smem) +
-                        (uint32_t)((wib * NS * OPS) * 32 + lane) * 16u;
+                        (uint32_t)((wib * NS) * 32 + lane) * 16u;
   const float init = (AGGR == PGH_MAX) ? -INFINITY : (AGGR == PGH_MIN) ? INFINITY : 0.f;
   for (int col = lane * 4; col < dense; col += 128) {
     const float* __restrict__ a_col = a_val + col;
-    const float* __restrict__ b_col = HAS_B ? b_val + col : nullptr;
     float* __restrict__ o_col = out + (size_t)r0 * ldo + col;
     float4 acc = make_float4(init, init, init, init);
     int cur = 0;
@@ -529,20 +422,19 @@ seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
     cur_end = __shfl_sync(kFull, rp, min(cur + 1, 31));                                 \
   } while (0)
     // plan registers: chunk holding the consume pointer (0) and the one after it (1)
-    int ci0 = 0, di0 = 0, ci1 = 0, di1 = 0;
+    int ci0 = 0, ci1 = 0;
     float sc0 = 1.f, sc1 = 1.f;
-#define PGH_LOAD_PLAN(BASE, CI, DI, SC)                                                 \
+#define PGH_LOAD_PLAN(BASE, CI, SC)                                                     \
   do {                                                                                  \
     const int t_ = (BASE) + lane;                                                       \
-    CI = 0; DI = 0; SC = 1.f;                                                           \
+    CI = 0; SC = 1.f;                                                                   \
     if (t_ < e_end) {                                                                   \
       CI = c ? __ldg(c + t_) : t_;                                                      \
-      if (HAS_B) DI = d ? __ldg(d + t_) : t_;                                           \
       if (a_scale) SC = __ldg(a_scale + CI);                                            \
     }                                                                                   \
   } while (0)
-    PGH_LOAD_PLAN(e_beg, ci0, di0, sc0);
-    PGH_LOAD_PLAN(e_beg + 32, ci1, di1, sc1);
+    PGH_LOAD_PLAN(e_beg, ci0, sc0);
+    PGH_LOAD_PLAN(e_beg + 32, ci1, sc1);
     int chunk_base = e_beg;                         // first entry of chunk 0's registers
     int ti = e_beg;                                 // next entry to issue
 // issue one commit group: entries ti .. ti+U-1 into the slots they map to
@@ -553,12 +445,8 @@ seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
       if (t_ < e_end) {                                                                 \
         const int off_ = t_ - chunk_base;                                               \
         const int cc_ = __shfl_sync(kFull, off_ < 32 ? ci0 : ci1, off_ & 31);           \
-        const uint32_t slot_ = ring + (uint32_t)((((t_ - e_beg) % NS) * OPS) * 512);    \
+        const uint32_t slot_ = ring + (uint32_t)(((t_ - e_beg) % NS) * 512);            \
         cp_async16(slot_, a_col + (size_t)cc_ * lda);                                   \
-        if (HAS_B) {                                                                    \
-          const int dd_ = __shfl_sync(kFull, off_ < 32 ? di0 : di1, off_ & 31);         \
-          cp_async16(slot_ + 512u, b_col + (size_t)dd_ * ldb);                          \
-        }                                                                               \
       }                                                                                 \
     }                                                                                   \
     cp_async_commit();                                                                  \
@@ -568,14 +456,13 @@ seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
     for (int g = 0; g < NG; ++g) PGH_ISSUE();
     for (int tc = e_beg; tc < e_end; tc += U) {
       cp_async_wait<NG - 1>();
-      float4 av[U], bv[U];
+      float4 av[U];
       float ss[U];
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int t = min(tc + u, e_end - 1);
-        const uint32_t slot = ring + (uint32_t)((((t - e_beg) % NS) * OPS) * 512);
+        const uint32_t slot = ring + (uint32_t)(((t - e_beg) % NS) * 512);
         av[u] = lds128(slot);
-        if (HAS_B) bv[u] = lds128(slot + 512u);
         ss[u] = a_scale ? __shfl_sync(kFull, sc0, (t - chunk_base) & 31) : 1.f;
       }
 #pragma unroll
@@ -587,9 +474,6 @@ seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
           if (a_scale)
             m = make_float4(__fmul_rn(m.x, ss[u]), __fmul_rn(m.y, ss[u]), __fmul_rn(m.z, ss[u]),
                             __fmul_rn(m.w, ss[u]));
-          if (HAS_B)
-            m = make_float4(__fmul_rn(m.x, bv[u].x), __fmul_rn(m.y, bv[u].y),
-                            __fmul_rn(m.z, bv[u].z), __fmul_rn(m.w, bv[u].w));
           if (AGGR == PGH_MAX)
             acc = make_float4(fmaxf(acc.x, m.x), fmaxf(acc.y, m.y), fmaxf(acc.z, m.z), fmaxf(acc.w, m.w));
           else if (AGGR == PGH_MIN)
@@ -604,8 +488,8 @@ seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
       PGH_ISSUE();
       if (tc + U - chunk_base >= 32) {              // consume pointer enters the next chunk
         chunk_base += 32;
-        ci0 = ci1; di0 = di1; sc0 = sc1;
-        PGH_LOAD_PLAN(chunk_base + 32, ci1, di1, sc1);
+        ci0 = ci1; sc0 = sc1;
+        PGH_LOAD_PLAN(chunk_base + 32, ci1, sc1);
       }
     }
     cp_async_wait<0>();
@@ -613,125 +497,6 @@ seg_gmr_ring_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
 #undef PGH_ISSUE
 #undef PGH_LOAD_PLAN
 #undef PGH_FLUSH
-  }
-}
-
-// ---------------------------------------------------------------------------------------
-// Staged variant (dense == 128, two operands, sum / mean): "shared-memory staging of each row's
-// key range" (BASELINE.json north_star).  For plans with many entries per output row -- the
-// 2-FWL key X___X___1___X___0, the sr25-shaped keys with ~12 entries per row, the I2 key -- the
-// lean kernel is bound by L1/L2 gather traffic: every operand row is fetched ~8-12 times.  Because
-// the tuple arrays are sorted by (root, node), the FIRST-operand rows that a tile of R consecutive
-// output rows touches lie in one short contiguous row range [lo, lo + cnt) (the tuples of the
-// roots the tile covers); that range is found once per batch (tile_range_kernel) and cached with
-// the plan.  A CTA copies the range into shared memory with coalesced 128-bit loads (each
-// first-operand row leaves L2 once per tile instead of once per entry) and its four warps then
-// reduce the tile's rows: first operand from shared memory, second operand gathered as before,
-// 4 entries = 4 independent 128-bit global loads in flight per lane.  Tiles whose range does not
-// fit (cnt > smax: e.g. groupings by the second operand, whose rows come from all over the batch)
-// read the first operand from global memory like the lean kernel.  Same sequential reduction
-// order per row as every other variant: deterministic, bit-identical results.
-constexpr int kStageThreads = 128;
-template <int AGGR, bool HAS_SCALE>
-__global__ void __launch_bounds__(kStageThreads)
-seg_gmr_staged_kernel(const float* __restrict__ a_val, const int* __restrict__ c,
-                      const float* __restrict__ a_scale, const float* __restrict__ b_val,
-                      const int* __restrict__ d, const int* __restrict__ rowptr, long long n_rows,
-                      int lda, int ldb, int ldo, int R, const int* __restrict__ tile_lo,
-                      const int* __restrict__ tile_cnt, int smax, int accum,
-                      float* __restrict__ out) {
-  extern __shared__ float4 stage[];                       // smax rows x 32 float4
-  constexpr unsigned kFull = 0xffffffffu;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const long long tile = blockIdx.x;
-  const int lo = __ldg(tile_lo + tile), cnt = __ldg(tile_cnt + tile);
-  const bool staged = cnt > 0 && cnt <= smax;
-  if (staged) {
-    const float* src = a_val + (size_t)lo * lda;
-    for (int idx = threadIdx.x; idx < cnt * 32; idx += kStageThreads)
-      stage[idx] = __ldg(reinterpret_cast<const float4*>(src + (size_t)(idx >> 5) * lda) + (idx & 31));
-    __syncthreads();
-  }
-  const long long r_end = min(n_rows, (tile + 1) * (long long)R);
-  const float* __restrict__ b_col = b_val + lane * 4;
-  const float* __restrict__ a_col = a_val + lane * 4;
-  for (long long r = tile * R + warp; r < r_end; r += kStageThreads / 32) {
-    const int e0 = __ldg(rowptr + r), e1 = __ldg(rowptr + r + 1);
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int base = e0; base < e1; base += 32) {
-      const int t = base + lane;
-      int ci = 0, di = 0;
-      float sc = 1.f;
-      if (t < e1) {
-        ci = c ? __ldg(c + t) : t;
-        di = d ? __ldg(d + t) : t;
-        if (HAS_SCALE) sc = __ldg(a_scale + ci);
-      }
-      const int chunk = min(32, e1 - base);
-      for (int k = 0; k < chunk; k += 4) {
-        float4 av[4], bv[4];
-        float ss[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const int kk = min(k + u, chunk - 1);            // clamped: loads stay unconditional
-          const int cc = __shfl_sync(kFull, ci, kk);
-          const int dd = __shfl_sync(kFull, di, kk);
-          bv[u] = __ldg(reinterpret_cast<const float4*>(b_col + (size_t)dd * ldb));
-          av[u] = staged ? stage[(cc - lo) * 32 + lane]
-                         : __ldg(reinterpret_cast<const float4*>(a_col + (size_t)cc * lda));
-          if (HAS_SCALE) ss[u] = __shfl_sync(kFull, sc, kk);
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          if (k + u < chunk) {
-            float4 m = av[u];
-            if (HAS_SCALE)
-              m = make_float4(__fmul_rn(m.x, ss[u]), __fmul_rn(m.y, ss[u]), __fmul_rn(m.z, ss[u]),
-                              __fmul_rn(m.w, ss[u]));
-            acc = make_float4(__fmaf_rn(m.x, bv[u].x, acc.x), __fmaf_rn(m.y, bv[u].y, acc.y),
-                              __fmaf_rn(m.z, bv[u].z, acc.z), __fmaf_rn(m.w, bv[u].w, acc.w));
-          }
-        }
-      }
-    }
-    if (AGGR == PGH_MEAN && e1 > e0) {
-      const float n_ = (float)(e1 - e0);
-      acc = make_float4(acc.x / n_, acc.y / n_, acc.z / n_, acc.w / n_);
-    }
-    float4* o = reinterpret_cast<float4*>(out + (size_t)r * ldo) + lane;
-    if (accum) {
-      const float4 p = *o;
-      acc = make_float4(__fadd_rn(p.x, acc.x), __fadd_rn(p.y, acc.y), __fadd_rn(p.z, acc.z),
-                        __fadd_rn(p.w, acc.w));
-    }
-    *o = acc;
-  }
-}
-
-// [lo, lo + cnt) = range of first-operand rows referenced by the entries of output rows
-// [tile * R, (tile + 1) * R); one warp per tile.  first == NULL: identity index.
-__global__ void tile_range_kernel(const int* __restrict__ rowptr, const int* __restrict__ first,
-                                  long long n_rows, int R, long long n_tiles,
-                                  int* __restrict__ lo, int* __restrict__ cnt) {
-  const long long tile = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (tile >= n_tiles) return;
-  const int e0 = __ldg(rowptr + tile * R);
-  const int e1 = __ldg(rowptr + min(n_rows, (tile + 1) * (long long)R));
-  int mn = 0x7fffffff, mx = -1;
-  for (int e = e0 + lane; e < e1; e += 32) {
-    const int v = first ? __ldg(first + e) : e;
-    mn = min(mn, v);
-    mx = max(mx, v);
-  }
-#pragma unroll
-  for (int s = 16; s >= 1; s >>= 1) {
-    mn = min(mn, __shfl_xor_sync(0xffffffffu, mn, s));
-    mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, s));
-  }
-  if (lane == 0) {
-    lo[tile] = e1 > e0 ? mn : 0;
-    cnt[tile] = e1 > e0 ? mx - mn + 1 : 0;
   }
 }
 
@@ -879,12 +644,6 @@ __global__ void seg_reduce_i64_kernel(const long long* __restrict__ val,
   out[i] = acc;
 }
 
-// test hook: PYGHO_B200_ROWWISE=1 keeps the row-per-lane-group kernel for every width
-static const bool g_force_rowwise = [] {
-  const char* e = getenv("PYGHO_B200_ROWWISE");
-  return e && e[0] == '1';
-}();
-
 struct Geometry {
   int vec, lpr;
   unsigned blocks;
@@ -905,63 +664,37 @@ static Geometry geometry(int64_t n_rows, int64_t dense, bool aligned) {
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 
-// run-time tuning knobs (pgh_set_tuning): [0] seg_gmr variant (-1 = built-in choice),
-// [1] ring kernel: target plan entries per warp, [6] profiling: no row stores
-// [2..5] fused BN kernels (fused_mlp.cu)
-int g_tune[16] = {-1, 16, 0, 0, 0, 0, 0, 0, /* [8] programmatic dependent launch */ 1, 0, 0, 0, 0, 0, 0, 0};
+// run-time tuning knobs (pgh_set_tuning): [2..5] fused BN kernels (fused_mlp.cu), [7] mamamm
+// profiling ablations (mamamm_smem.cu), [8] programmatic dependent launch (common.cuh)
+int g_tune[16] = {0, 0, 0, 0, 0, 0, 0, 0, /* [8] */ 1, 0, 0, 0, 0, 0, 0, 0};
 
-template <int AGGR, bool HAS_B, int NS, int U, int WARPS>
-static void launch_ring_t(cudaStream_t s, const float* a_val, const int* c, const float* a_scale,
-                          const float* b_val, const int* d, const int* rowptr, int64_t n_rows,
-                          int dense, int lda, int ldb, int ldo, int rw, int accum, float* out) {
-  constexpr int smem = WARPS * NS * (HAS_B ? 2 : 1) * 512;
-  auto kern = seg_gmr_ring_kernel<AGGR, HAS_B, NS, U, WARPS>;
+// single operand (pooling, unpooling, coalesce): the cp.async ring kernel wins
+// (profiles/probes/bench_gmr.py.txt) with 8 stages of 2 entries and 4 warps per CTA
+template <int AGGR>
+static void launch_ring(cudaStream_t s, const float* a_val, const int* c, const float* a_scale,
+                        const int* rowptr, int64_t n_rows, int64_t n_entries, int dense, int lda,
+                        int ldo, int accum, float* out) {
+  constexpr int NS = 8, U = 2, WARPS = 4;
+  constexpr int kEntriesPerWarp = 16;               // rows per warp: aim at this many plan entries
+  constexpr int smem = WARPS * NS * 512;
+  int rw = kEntriesPerWarp;
+  if (n_entries > 0 && n_rows > 0) {
+    const double avg = (double)n_entries / (double)n_rows;
+    rw = (int)((double)kEntriesPerWarp / (avg > 0.5 ? avg : 0.5));
+  }
+  if (rw < 1) rw = 1;
+  if (rw > 31) rw = 31;
+  auto kern = seg_gmr_ring_kernel<AGGR, NS, U, WARPS>;
   static bool configured = false;
   if (!configured) {
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     configured = true;
   }
   const unsigned nb = blocks_for(n_rows, WARPS * rw);
-  launch_pdl(kern, dim3(nb), dim3(WARPS * 32), smem, s, a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb,
-                                    ldo, rw, accum, out);
+  launch_pdl(kern, dim3(nb), dim3(WARPS * 32), smem, s, a_val, c, a_scale, nullptr, nullptr, rowptr,
+             n_rows, dense, lda, 0, ldo, rw, accum, out);
 }
 
-template <int AGGR>
-static void launch_ring(int variant, cudaStream_t s, const float* a_val, const int* c,
-                        const float* a_scale, const float* b_val, const int* d,
-                        const int* rowptr, int64_t n_rows, int64_t n_entries, int dense, int lda,
-                        int ldb, int ldo, int accum, float* out) {
-  int rw = 16;
-  if (n_entries > 0 && n_rows > 0) {
-    const double avg = (double)n_entries / (double)n_rows;
-    rw = (int)((double)g_tune[1] / (avg > 0.5 ? avg : 0.5));
-  }
-  if (rw < 1) rw = 1;
-  if (rw > 31) rw = 31;
-#define PGH_RING(NS, U, W)                                                                   \
-  do {                                                                                       \
-    if (b_val) launch_ring_t<AGGR, true, NS, U, W>(s, a_val, c, a_scale, b_val, d, rowptr,   \
-                                                   n_rows, dense, lda, ldb, ldo, rw, accum,  \
-                                                   out);                                     \
-    else launch_ring_t<AGGR, false, NS, U, W>(s, a_val, c, a_scale, b_val, d, rowptr,        \
-                                              n_rows, dense, lda, ldb, ldo, rw, accum, out); \
-  } while (0)
-  switch (variant) {
-    case 11: PGH_RING(8, 4, 8); break;
-    case 12: PGH_RING(8, 2, 8); break;
-    case 13: PGH_RING(8, 2, 4); break;
-    case 14: PGH_RING(4, 2, 8); break;
-    case 15: PGH_RING(4, 2, 4); break;
-    case 16: PGH_RING(8, 1, 4); break;
-    case 17: PGH_RING(16, 2, 8); break;
-    case 18: PGH_RING(4, 4, 8); break;
-    default: PGH_RING(16, 4, 4); break;
-  }
-#undef PGH_RING
-}
-
-
-// variants 30..: lean streaming kernel (see seg_gmr_lean_kernel)
 struct LeanExtra {                       // optional fused epilogue work, all row-aligned with out
   const float* add_src = nullptr;        // out = add_src + reduction (NULL + accum: in place)
   int ld_add = 0;
@@ -973,17 +706,31 @@ struct LeanExtra {                       // optional fused epilogue work, all ro
   int ld_copy_dst = 0;
 };
 
-template <int AGGR, int U, int MINB>
+// two operands or a fused epilogue: the lean kernel (half the instructions of the first
+// streaming kernel, 54 vs 61 us on the SSWL key, profiles/r1_gmr_ablate.txt) with 4 entries in
+// flight at 64 registers (4 CTAs/SM), measured best for the short rows of the SSWL keys
+template <int AGGR>
 static void launch_lean(cudaStream_t s, const float* a_val, const int* c, const float* a_scale,
                         const float* b_val, const int* d, const int* rowptr, int64_t n_rows,
-                        int dense, int lda, int ldb, int ldo, int rw, int accum, float* out,
-                        const LeanExtra& x) {
+                        int64_t n_entries, int dense, int lda, int ldb, int ldo, int accum,
+                        float* out, const LeanExtra& x) {
+  // rows per warp: aim at ~32 plan entries per warp, at least 4 warps' worth of blocks per SM
+  int rw = kMaxRW;
+  if (n_entries > 0 && n_rows > 0) {
+    const double avg = (double)n_entries / (double)n_rows;
+    rw = (int)(32.0 / (avg > 0.5 ? avg : 0.5));
+    // small problems: keep >= 4 CTAs per SM in the grid rather than long per-warp streams
+    const int64_t cap = n_rows / (int64_t)(kSMs * 4 * (kThreads / 32));
+    if (rw > cap) rw = (int)cap;
+    if (rw < 1) rw = 1;
+    if (rw > kMaxRW) rw = kMaxRW;
+  }
   const unsigned nb = blocks_for(n_rows, (kThreads / 32) * rw);
   const float* acc_src = x.add_src ? x.add_src : out;
   const int lds = x.add_src ? x.ld_add : ldo;
   const bool acc = accum || x.add_src;
 #define PGH_LEAN(B, S, A)                                                                      \
-  launch_pdl(seg_gmr_lean_kernel<AGGR, B, S, A, U, MINB>, dim3(nb), dim3(kThreads), 0, s,                          \
+  launch_pdl(seg_gmr_lean_kernel<AGGR, B, S, A, 4, 4>, dim3(nb), dim3(kThreads), 0, s,         \
       a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, acc_src, lds,     \
       x.add_src2, x.ld_add2, x.copy_src, x.ld_copy_src, x.copy_dst, x.ld_copy_dst, out)
   const int sel = (b_val ? 4 : 0) | (a_scale ? 2 : 0) | (acc ? 1 : 0);
@@ -1000,68 +747,21 @@ static void launch_lean(cudaStream_t s, const float* a_val, const int* c, const 
 #undef PGH_LEAN
 }
 
+// dense % 128 == 0 with 16-byte rows: the ring kernel for one operand, the lean kernel for two
+// operands or a fused epilogue; any other width or alignment: the row-wise kernel
 template <int AGGR, int VEC>
 static int launch_gmr(const Geometry& g, cudaStream_t s, const float* a_val, const int* c,
                       const float* a_scale, const float* b_val, const int* d,
                       const int* rowptr, int64_t n_rows, int64_t n_entries, int dense, int lda,
                       int ldb, int ldo, int accum, float* out, const LeanExtra* extra = nullptr) {
-  if (VEC == 4 && dense % 128 == 0 && !g_force_rowwise) {
-    // rows per warp: aim at ~32 plan entries per warp, at least 4 warps' worth of blocks per SM
-    int rw = kMaxRW;
-    if (n_entries > 0 && n_rows > 0) {
-      const double avg = (double)n_entries / (double)n_rows;
-      rw = (int)(32.0 / (avg > 0.5 ? avg : 0.5));
-      // small problems: keep >= 4 CTAs per SM in the grid rather than long per-warp streams
-      const int64_t cap = n_rows / (int64_t)(kSMs * 4 * (kThreads / 32));
-      if (rw > cap) rw = (int)cap;
-      if (rw < 1) rw = 1;
-      if (rw > kMaxRW) rw = kMaxRW;
-    }
-    const unsigned nb = blocks_for(n_rows, (kThreads / 32) * rw);
-    if (g_tune[6] == 1) accum = 2;                  // profiling only: no row stores (WRONG results)
-    // measured on B200 (profiles/README.md): 4 entries in flight at 64 registers (4 CTAs/SM)
-    // is best for the short rows of the SSWL keys, 2 entries at 48 registers (5 CTAs/SM) for
-    // long rows (the 2-FWL key, ~8 entries per row); PYGHO_B200_GMR_VARIANT overrides
-    static const int forced = [] { const char* e = getenv("PYGHO_B200_GMR_VARIANT"); return e ? atoi(e) : -1; }();
-    int variant = g_tune[0] >= 0 ? g_tune[0] : forced;
-    // single operand (pooling, unpooling, coalesce): the cp.async ring wins (bench_gmr.py);
-    // two operands: the lean kernel (half the instructions of the first streaming kernel,
-    // 54 vs 61 us on the SSWL key, profiles/r1_gmr_ablate.txt)
-    if (variant < 0) variant = b_val ? 30 : 13;
-    if (extra && variant < 30) variant = 30;        // the fused epilogue lives in the lean kernels
-    if (variant >= 30) {
-      if (g_tune[6] == 1) accum = 0;
+  if (VEC == 4 && dense % 128 == 0) {
+    if (b_val || extra) {
       const LeanExtra none;
-      const LeanExtra& x = extra ? *extra : none;
-      if (variant == 31) launch_lean<AGGR, 8, 2>(s, a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out, x);
-      else if (variant == 32) launch_lean<AGGR, 2, 5>(s, a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out, x);
-      else if (variant == 33) launch_lean<AGGR, 4, 3>(s, a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out, x);
-      else launch_lean<AGGR, 4, 4>(s, a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out, x);
-      return 0;
-    }
-    if (variant >= 20)      // 20-25 (bulk copy) and 34/35 (register pipelining) were round-1
-      variant = 13;         // negative results: archived under profiles/probes/, not shipped
-    if (variant >= 10) {
-      launch_ring<AGGR>(variant, s, a_val, c, a_scale, b_val, d, rowptr, n_rows, n_entries, dense, lda, ldb, ldo, accum, out);
-      return 0;
-    }
-    if (variant < 0) variant = (n_entries > 6 * n_rows) ? 3 : 2;
-    if (b_val) {
-      if (variant == 1)
-        launch_pdl(seg_gmr_stream_kernel<AGGR, true, 8, 1>, dim3(nb), dim3(kThreads), 0, s, 
-            a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out);
-      else if (variant == 2)
-        launch_pdl(seg_gmr_stream_kernel<AGGR, true, 4, 4>, dim3(nb), dim3(kThreads), 0, s, 
-            a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out);
-      else if (variant == 3)
-        launch_pdl(seg_gmr_stream_kernel<AGGR, true, 2, 5>, dim3(nb), dim3(kThreads), 0, s, 
-            a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out);
-      else
-        launch_pdl(seg_gmr_stream_kernel<AGGR, true, 4, 1>, dim3(nb), dim3(kThreads), 0, s, 
-            a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out);
+      launch_lean<AGGR>(s, a_val, c, a_scale, b_val, d, rowptr, n_rows, n_entries, dense, lda, ldb,
+                        ldo, accum, out, extra ? *extra : none);
     } else {
-      launch_pdl(seg_gmr_stream_kernel<AGGR, false, 8, 1>, dim3(nb), dim3(kThreads), 0, s, 
-          a_val, c, a_scale, b_val, d, rowptr, n_rows, dense, lda, ldb, ldo, rw, accum, out);
+      launch_ring<AGGR>(s, a_val, c, a_scale, rowptr, n_rows, n_entries, dense, lda, ldo, accum,
+                        out);
     }
     return 0;
   }
@@ -1080,10 +780,10 @@ static int launch_gmr(const Geometry& g, cudaStream_t s, const float* a_val, con
 using namespace pgh;
 
 extern "C" const char* pgh_last_error(void) { return pgh::g_err; }
-extern "C" int pgh_abi_version(void) { return 3; }
+extern "C" int pgh_abi_version(void) { return 4; }
 
 extern "C" int pgh_set_tuning(int key, int value) {
-  if (key < 0 || key >= 16) return arg_error("set_tuning: key");
+  if (!((key >= 2 && key <= 5) || key == 7 || key == 8)) return arg_error("set_tuning: key");
   pgh::g_tune[key] = value;
   return 0;
 }
@@ -1183,56 +883,6 @@ extern "C" int pgh_seg_gmr_fused_f32(const float* a_val, int64_t lda, const int3
   return check_launch("seg_gmr_fused");
 }
 
-extern "C" int pgh_tile_ranges(const int32_t* rowptr, const int32_t* first, int64_t n_rows,
-                               int64_t rows_per_tile, int32_t* tile_lo, int32_t* tile_cnt,
-                               void* stream) {
-  if (!rowptr || !tile_lo || !tile_cnt || n_rows < 0 || rows_per_tile < 1 || rows_per_tile > (1 << 20))
-    return arg_error("tile_ranges: arguments");
-  if (n_rows == 0) return 0;
-  const long long n_tiles = (n_rows + rows_per_tile - 1) / rows_per_tile;
-  tile_range_kernel<<<blocks_for(n_tiles * 32, 256), 256, 0, as_stream(stream)>>>(
-      rowptr, first, n_rows, (int)rows_per_tile, n_tiles, tile_lo, tile_cnt);
-  return check_launch("tile_ranges");
-}
-
-extern "C" int pgh_seg_gmr_staged_f32(const float* a_val, int64_t lda, const int32_t* c,
-                                      const float* a_scale, const float* b_val, int64_t ldb,
-                                      const int32_t* d, const int32_t* rowptr, int64_t n_rows,
-                                      int64_t dense, int aggr, int accumulate,
-                                      const int32_t* tile_lo, const int32_t* tile_cnt,
-                                      int64_t rows_per_tile, int64_t max_stage_rows, float* out,
-                                      int64_t ldo, void* stream) {
-  if (!a_val || !b_val || !rowptr || !tile_lo || !tile_cnt || !out)
-    return arg_error("seg_gmr_staged: null pointer (two operands and a CSR grouping are required)");
-  if (dense != 128) return arg_error("seg_gmr_staged: dense must be 128");
-  if (aggr < 0 || aggr > 1) return arg_error("seg_gmr_staged: sum or mean only");
-  if (rows_per_tile < 1 || max_stage_rows < 1 || max_stage_rows > 256)
-    return arg_error("seg_gmr_staged: tile geometry");
-  const int64_t lim = 0x7fffffff;
-  if (lda < dense || ldb < dense || ldo < dense || lda > lim || ldb > lim || ldo > lim || lda % 4 ||
-      ldb % 4 || ldo % 4 || !aligned16(a_val) || !aligned16(b_val) || !aligned16(out))
-    return arg_error("seg_gmr_staged: rows must be 16-byte aligned");
-  if (n_rows <= 0) return 0;
-  const long long n_tiles = (n_rows + rows_per_tile - 1) / rows_per_tile;
-  const size_t smem = (size_t)max_stage_rows * 512;
-  cudaStream_t s = as_stream(stream);
-#define PGH_STAGED(AG, SC)                                                                          \
-  do {                                                                                              \
-    static size_t set_ = 0;                                                                         \
-    if (smem > set_) {                                                                              \
-      PGH_CUDA(cudaFuncSetAttribute(seg_gmr_staged_kernel<AG, SC>,                                  \
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));       \
-      set_ = smem;                                                                                  \
-    }                                                                                               \
-    seg_gmr_staged_kernel<AG, SC><<<(unsigned)n_tiles, kStageThreads, smem, s>>>(                   \
-        a_val, c, a_scale, b_val, d, rowptr, n_rows, (int)lda, (int)ldb, (int)ldo,                  \
-        (int)rows_per_tile, tile_lo, tile_cnt, (int)max_stage_rows, accumulate, out);               \
-  } while (0)
-  if (aggr == PGH_SUM) { if (a_scale) PGH_STAGED(PGH_SUM, true); else PGH_STAGED(PGH_SUM, false); }
-  else { if (a_scale) PGH_STAGED(PGH_MEAN, true); else PGH_STAGED(PGH_MEAN, false); }
-#undef PGH_STAGED
-  return check_launch("seg_gmr_staged");
-}
 
 extern "C" int pgh_seg_gmr_f32(const float* a_val, const int32_t* c, const float* a_scale,
                                const float* b_val, const int32_t* d, const int32_t* rowptr,

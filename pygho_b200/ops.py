@@ -165,36 +165,6 @@ def _seg_gmr_fused_fake(a_val, c, a_scale, b_val, d, rowptr, n_rows, aggr, add_s
     return None
 
 
-_LIB.define("seg_gmr_staged(Tensor a_val, Tensor? c, Tensor? a_scale, Tensor b_val, Tensor? d, "
-            "Tensor rowptr, int n_rows, int aggr, Tensor tile_lo, Tensor tile_cnt, int rows_per_tile, "
-            "int max_stage_rows) -> Tensor")
-
-
-def _seg_gmr_staged_cuda(a_val, c, a_scale, b_val, d, rowptr, n_rows, aggr, tile_lo, tile_cnt,
-                         rows_per_tile, max_stage_rows):
-    """seg_gmr with the first operand's row range of every tile staged in shared memory
-    (dense == 128, two operands, sum / mean); results equal ``seg_gmr`` bit for bit."""
-    a_val, b_val, a_scale = _rows2d(a_val), _rows2d(b_val), _f32c(a_scale)
-    c, d, rowptr = _i32c(c), _i32c(d), _i32c(rowptr)
-    out = torch.empty((n_rows, a_val.shape[1]), dtype=torch.float32, device=a_val.device)
-    if n_rows:
-        call("pgh_seg_gmr_staged_f32", ptr(a_val), a_val.stride(0), ptr(c), ptr(a_scale), ptr(b_val),
-             b_val.stride(0), ptr(d), ptr(rowptr), n_rows, a_val.shape[1], aggr, 0, ptr(_i32c(tile_lo)),
-             ptr(_i32c(tile_cnt)), rows_per_tile, max_stage_rows, ptr(out), out.stride(0),
-             stream_ptr(a_val.device))
-        _lib.count_launch()
-    return out
-
-
-_LIB.impl("seg_gmr_staged", _seg_gmr_staged_cuda, "CUDA")
-
-
-@torch.library.register_fake("pygho_b200::seg_gmr_staged")
-def _seg_gmr_staged_fake(a_val, c, a_scale, b_val, d, rowptr, n_rows, aggr, tile_lo, tile_cnt,
-                         rows_per_tile, max_stage_rows):
-    return a_val.new_empty((n_rows, a_val.shape[1]))
-
-
 _LIB.define("seg_tie_scale(Tensor a_val, Tensor? c, Tensor? b_val, Tensor? d, Tensor? rowptr, "
             "Tensor out, Tensor grad) -> Tensor")
 
@@ -711,27 +681,10 @@ _ops = torch.ops.pygho_b200
 
 
 # ------------------------------------------------------------------------- autograd
-# The staged kernel is correct (bit-identical) but measured SLOWER than the streaming kernels on a
-# B200 -- 248 vs 127 us on the ZINC 2-FWL key, 64 vs 34 us on sr25 X.A, 529 vs 318 us on the I2 key
-# (profiles/r2_staged_kernel.md): L1 already serves half of the repeated first-operand rows, and
-# the staging phase + 48 KB of shared memory per CTA cost more latency hiding than the saved L2
-# requests return.  Opt-in (PYGHO_B200_STAGED=1) until it overlaps staging with the reduction.
-_STAGED = os.environ.get("PYGHO_B200_STAGED", "0") == "1"
-
-
 def _gmr(plan, which: str, first_val: Tensor, scale: Optional[Tensor], second_val: Optional[Tensor],
          n_rows: int, aggr: int) -> Tensor:
-    """One segmented reduce over grouping ``which`` of ``plan``: the staged kernel when the plan
-    has enough reuse of the first operand's rows (plans.TriplePlan.tiles), else the streaming
-    kernels."""
+    """One segmented reduce over grouping ``which`` of ``plan``."""
     g = plan.group(which)
-    if (_STAGED and second_val is not None and aggr <= 1 and first_val.ndim == 2
-            and first_val.shape[1] == 128 and second_val.shape[0] > 0 and first_val.shape[0] > 0):
-        t = plan.tiles(which)
-        if t is not None:
-            return _ops.seg_gmr_staged(first_val, g.first, scale, second_val, g.second, g.rowptr,
-                                       n_rows, aggr, t[0], t[1], plan.STAGE_ROWS_PER_TILE,
-                                       plan.STAGE_MAX_ROWS)
     return _ops.seg_gmr(first_val, g.first, scale, second_val,
                         g.second if second_val is not None else None, g.rowptr, n_rows, aggr)
 

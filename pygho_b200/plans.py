@@ -154,7 +154,6 @@ class TriplePlan:
         self._groups: Dict[str, Group] = {}
         self._inv: Optional[Tensor] = None
         self._swapped: Optional["TriplePlan"] = None
-        self._tiles: Dict[str, Optional[Tuple[Tensor, Tensor]]] = {}
 
     _ORDER = {"a": ("c", "d", "n_out"), "c": ("a", "d", "n_a"), "d": ("a", "c", "n_b")}
 
@@ -170,34 +169,6 @@ class TriplePlan:
                 g = Group(rowptr, _take(self.idx[first], perm), _take(self.idx[second], perm))
             self._groups[which] = g
         return g
-
-    STAGE_ROWS_PER_TILE = 32      # output rows per CTA tile of the staged kernel
-    STAGE_MAX_ROWS = 96           # first-operand rows staged per tile (48 KB of shared memory)
-
-    def tiles(self, which: str) -> Optional[Tuple[Tensor, Tensor]]:
-        """(tile_lo, tile_cnt) int32 for the staged segmented-reduce kernel on grouping ``which``
-        (see csrc/seg_gmr.cu ``seg_gmr_staged_kernel``), or None when staging does not pay:
-        fewer than ~4 entries per row (each first-operand row is reused too rarely), or fewer than
-        80 % of the tiles have a first-operand row range that fits in shared memory (e.g. the
-        grouping by the second operand, whose rows come from all over the batch).  Decided once
-        per plan and grouping (one host read-back, like the plan builders) and cached."""
-        if which in self._tiles:
-            return self._tiles[which]
-        g = self.group(which)
-        n_rows = getattr(self, self._ORDER[which][2])
-        res = None
-        if g.rowptr is not None and n_rows > 0 and self.T >= 4 * n_rows:
-            R = self.STAGE_ROWS_PER_TILE
-            n_tiles = (n_rows + R - 1) // R
-            lo = _empty(n_tiles, torch.int32, g.rowptr.device)
-            cnt = _empty(n_tiles, torch.int32, g.rowptr.device)
-            _launch("pgh_tile_ranges", ptr(g.rowptr), ptr(g.first), n_rows, R, ptr(lo), ptr(cnt),
-                    stream_ptr(g.rowptr.device))
-            fits = float((cnt <= self.STAGE_MAX_ROWS).float().mean().item())
-            if fits >= 0.8:
-                res = (lo, cnt)
-        self._tiles[which] = res
-        return res
 
     def inv_count(self) -> Tensor:
         """1 / max(#triples of each output row, 1): the mean-backward scale."""

@@ -226,17 +226,6 @@ class _Mirror:
             self.obj(d._groups[which], s.group(which), dd_src)
         if d._inv is not None:
             self.tensor(d._inv, s.inv_count(), dd_src)
-        for which, t in getattr(d, "_tiles", {}).items():
-            if t is not None:          # the template decided to stage: the fresh batch follows it
-                g = s.group(which)
-                n_rows = getattr(s, s._ORDER[which][2])
-                n_tiles = (n_rows + s.STAGE_ROWS_PER_TILE - 1) // s.STAGE_ROWS_PER_TILE
-                lo = torch.empty((n_tiles,), dtype=torch.int32, device=g.rowptr.device)
-                cnt = torch.empty_like(lo)
-                P._launch("pgh_tile_ranges", P.ptr(g.rowptr), P.ptr(g.first), n_rows,
-                          s.STAGE_ROWS_PER_TILE, P.ptr(lo), P.ptr(cnt), P.stream_ptr(lo.device))
-                self.tensor(t[0], lo, dd_src)
-                self.tensor(t[1], cnt, dd_src)
         if d._swapped is not None:
             self.plan(d._swapped, s.swapped(), dd_src)
         t = getattr(d, "_transposed", None)
@@ -259,7 +248,6 @@ class _Mirror:
                 o._groups = {}
                 o._swapped = None
                 o._inv = None
-                o._tiles = {}
                 if hasattr(o, "_transposed"):
                     o._transposed = None
         self.src_objs = []
@@ -337,7 +325,6 @@ def release_datadict(dd: Optional[dict]) -> None:
             subs = list(o.idx.values()) + list(dict.values(o._groups)) + [o._swapped, o._inv,
                                                                        getattr(o, "_transposed", None)]
             o._groups, o._swapped, o._inv = {}, None, None
-            o._tiles = {}
             if hasattr(o, "_transposed"):
                 o._transposed = None
             for v in subs:

@@ -32,7 +32,7 @@ def test_binding_table_matches_header():
     from pygho_b200 import _lib
     assert sorted(_lib.SIGNATURES) == _declared()
     lib = _lib.load()
-    assert lib.pgh_abi_version() == 3
+    assert lib.pgh_abi_version() == 4
     assert lib.pgh_last_error() is not None
 
 
@@ -52,6 +52,8 @@ def test_argument_errors_are_reported():
         _lib.call("pgh_seg_gmr_f32", None, None, None, None, None, None, 4, 0, 8, 0, None, None)
     with pytest.raises(_lib.KernelError, match="aggr"):
         _lib.call("pgh_seg_gmr_f32", 16, None, None, None, None, None, 4, 0, 8, 9, 16, None)
+    with pytest.raises(_lib.KernelError, match="set_tuning: key"):
+        _lib.call("pgh_set_tuning", 0, 2)
 
 
 def test_api_surface_names():
