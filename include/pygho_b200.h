@@ -377,6 +377,23 @@ int pgh_i2_emit(const uint8_t* D, const int64_t* edge_src, const int64_t* edge_d
 int pgh_spd_dense_i64(const uint8_t* D, const int64_t* node_ptr, const int64_t* sq_ptr,
                       int64_t n_graphs, int64_t nmax, int clamp, int64_t fill, int64_t* out,
                       uint8_t* mask, void* stream);
+/* Resistance distances of every graph of a block-diagonal batch, one CTA per graph:
+ *   R[sq_ptr[g] + i*n_g + j] = L+[i,i] + L+[j,j] - 2 L+[i,j]   (float32, the layout of D above)
+ * with L+ the Moore-Penrose pseudo-inverse of the combinatorial Laplacian of the SIMPLE
+ * undirected graph (both edge directions count once, duplicates once, self-loops dropped:
+ * spdsampler's directed=False).  Pairs in different components get L+[i,i] + L+[j,j]; an
+ * isolated node has L+[i,i] = 0.  fp64 inversion in shared memory (n_g(n_g+1) doubles plus the
+ * bit-set adjacency), so graphs of 1..128 nodes; R is bit-symmetric with an exact 0 diagonal.
+ * Replaces the per-graph pinv of rdsampler (MaTupleSampler.py:34-57).                         */
+int pgh_resistance_f32(const int64_t* edge_src, const int64_t* edge_dst, const int64_t* node_ptr,
+                       const int64_t* edge_ptr, const int64_t* sq_ptr, int64_t n_graphs,
+                       int64_t max_nodes, float* R, void* stream);
+/* rdsampler's padding (MaTupleSampler.py:34-57 + to_dense_tuplefeat, MaData.py:152-212):
+ * out (B, nmax, nmax) = R of pgh_resistance_f32 where mask = (i < n_g) & (j < n_g), `fill`
+ * elsewhere.                                                                                  */
+int pgh_rd_dense_f32(const float* R, const int64_t* node_ptr, const int64_t* sq_ptr,
+                     int64_t n_graphs, int64_t nmax, float fill, float* out, uint8_t* mask,
+                     void* stream);
 /* to_dense_x (MaData.py:109-149): out[g, i, :] = src[ptr[g] + i, :] for i < n_g, `fill`
  * elsewhere; mask[g, i] = i < n_g.  Elements are copied as raw 4- or 8-byte words
  * (elem_bytes), fill is the raw bit pattern.                                                  */

@@ -85,6 +85,8 @@ SIGNATURES = {
     "pgh_i2_count": (_i, [_p, _p, _p, _p, _p, _p, _i64, _i, _p, _p]),
     "pgh_i2_emit": (_i, [_p, _p, _p, _p, _p, _p, _p, _i64, _i64, _i, _p, _p, _p]),
     "pgh_spd_dense_i64": (_i, [_p, _p, _p, _i64, _i64, _i, _i64, _p, _p, _p]),
+    "pgh_resistance_f32": (_i, [_p, _p, _p, _p, _p, _i64, _i64, _p, _p]),
+    "pgh_rd_dense_f32": (_i, [_p, _p, _p, _i64, _i64, _f, _p, _p, _p]),
     "pgh_pad_rows": (_i, [_p, _p, _i64, _i64, _i64, _i, _u64, _p, _p, _p]),
     "pgh_dense_adj": (_i, [_p, _p, _p, _p, _p, _i64, _i64, _i64, _i64, _i, _u64, _p, _p, _p]),
 }

@@ -11,7 +11,9 @@
 //                level is |frontier| shared-memory row ORs and no global traffic at all.
 //   khop_emit  : one warp per root node compacts its distance row with ballots into the
 //                (i, j)-sorted tuple list at the offset given by the scanned row counts.
-//   spd_dense / pad_rows / dense_adj : one thread per output element, coalesced stores.
+//   resistance : one CTA per graph (n <= 128); fp64 Gauss-Jordan inversion of the grounded
+//                Laplacian in shared memory (<= 132 KiB), the only floating-point kernel here.
+//   spd_dense / rd_dense / pad_rows / dense_adj : one thread per output element, coalesced.
 #include "common.cuh"
 
 namespace pgh {
@@ -174,6 +176,139 @@ i2_edge_kernel(const unsigned char* __restrict__ D, const long long* __restrict_
   if (!EMIT && lane == 0) cnt[e] = total;
 }
 
+// rdsampler (hodata/MaTupleSampler.py:34-57): effective resistance of every node pair,
+// R[i, j] = L+[i, i] + L+[j, j] - 2 L+[i, j] with L+ the pseudo-inverse of the Laplacian of the
+// simple undirected graph.  One CTA per graph, all in shared memory:
+//   adjacency bit set (both directions, duplicates once, no self-loops) -> degrees and connected
+//   components (min-label propagation) -> M = L + sum_c (1/n_c) 1_c 1_c^T, which is SPD and has
+//   M^-1 = L+ + sum_c (1/n_c) 1_c 1_c^T -> in-place Gauss-Jordan inversion of M in fp64 (no
+//   pivoting: SPD) -> R from M^-1, where the 1/n_c terms cancel within a component and are
+//   subtracted across components.  Every value is computed from the ordered pair (min, max), so
+//   R is bit-symmetric; the diagonal is written as 0.
+constexpr int kRdThreads = 256;
+constexpr int kRdMaxNodes = 128;
+
+inline size_t rd_smem_bytes(int n) {
+  const int W = (n + 31) >> 5;
+  return (size_t)n * (n + 1) * sizeof(double)                  // M (n x n) + pivot column
+         + (size_t)n * W * sizeof(unsigned int)               // adjacency bits
+         + (size_t)2 * n * sizeof(int);                        // component label, component size
+}
+
+__global__ void __launch_bounds__(kRdThreads)
+resistance_kernel(const long long* __restrict__ edge_src, const long long* __restrict__ edge_dst,
+                  const long long* __restrict__ node_ptr, const long long* __restrict__ edge_ptr,
+                  const long long* __restrict__ sq_ptr, int max_nodes, float* __restrict__ R) {
+  extern __shared__ double rd_smem[];
+  const int g = blockIdx.x;
+  const long long n0 = node_ptr[g];
+  const int n = (int)(node_ptr[g + 1] - n0);
+  if (n <= 0 || n > max_nodes) return;                // host checked max_nodes; stay in bounds
+  const int W = (n + 31) >> 5;
+  const int nn = n * n;
+  double* M = rd_smem;                                 // M[i * n + j]
+  double* col = M + nn;                                // pivot column of the current step
+  unsigned int* adj = reinterpret_cast<unsigned int*>(col + n);   // adj[i * W + w]
+  int* label = reinterpret_cast<int*>(adj + n * W);
+  int* csize = label + n;
+
+  for (int i = threadIdx.x; i < n * W; i += blockDim.x) adj[i] = 0u;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    label[i] = i;
+    csize[i] = 0;
+  }
+  __syncthreads();
+  const long long e0 = edge_ptr[g], e1 = edge_ptr[g + 1];
+  for (long long e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
+    const long long s = edge_src[e] - n0, t = edge_dst[e] - n0;
+    if (s >= 0 && s < n && t >= 0 && t < n && s != t) {
+      atomicOr(&adj[(int)s * W + (int)(t >> 5)], 1u << (int)(t & 31));
+      atomicOr(&adj[(int)t * W + (int)(s >> 5)], 1u << (int)(s & 31));
+    }
+  }
+  __syncthreads();
+
+  // connected components: every node takes the smallest label of its closed neighbourhood until
+  // nothing changes; the fixed point is the smallest node id of the component
+  const int v = threadIdx.x;
+  while (true) {
+    int m = v < n ? label[v] : 0;
+    if (v < n)
+      for (int w = 0; w < W; ++w)
+        for (unsigned int bits = adj[v * W + w]; bits; bits &= bits - 1)
+          m = min(m, label[(w << 5) + __ffs(bits) - 1]);
+    __syncthreads();
+    const bool changed = v < n && m != label[v];
+    if (changed) label[v] = m;
+    if (!__syncthreads_or(changed)) break;
+  }
+  if (v < n) atomicAdd(&csize[label[v]], 1);
+  __syncthreads();
+
+  for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+    const int i = idx / n, j = idx - i * n;
+    double x = 0.0;
+    if (i == j) {
+      for (int w = 0; w < W; ++w) x += (double)__popc(adj[i * W + w]);
+    } else if ((adj[i * W + (j >> 5)] >> (j & 31)) & 1u) {
+      x = -1.0;
+    }
+    if (label[i] == label[j]) x += 1.0 / (double)csize[label[i]];
+    M[idx] = x;
+  }
+  __syncthreads();
+
+  // in-place Gauss-Jordan, one warp per row: after step k, M holds the inverse with respect to
+  // pivots 0..k.  Each element sees the same operations in the same order on every launch.
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+  for (int k = 0; k < n; ++k) {
+    for (int i = threadIdx.x; i < n; i += blockDim.x) col[i] = M[i * n + k];
+    __syncthreads();
+    const double piv = 1.0 / col[k];
+    for (int j = threadIdx.x; j < n; j += blockDim.x) M[k * n + j] = j == k ? piv : M[k * n + j] * piv;
+    __syncthreads();
+    for (int i = warp; i < n; i += nwarps) {
+      if (i == k) continue;
+      const double f = col[i];
+      for (int j = lane; j < n; j += 32)
+        M[i * n + j] = j == k ? -f * piv : M[i * n + j] - f * M[k * n + j];
+    }
+    __syncthreads();
+  }
+
+  float* __restrict__ Rg = R + sq_ptr[g];
+  for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+    const int r = idx / n, c = idx - r * n;
+    const int i = min(r, c), j = max(r, c);
+    float out = 0.0f;
+    if (i != j) {
+      double x;
+      if (label[i] == label[j])
+        x = M[i * n + i] + M[j * n + j] - 2.0 * M[i * n + j];
+      else
+        x = (M[i * n + i] - 1.0 / (double)csize[label[i]]) +
+            (M[j * n + j] - 1.0 / (double)csize[label[j]]);
+      out = (float)x;
+    }
+    Rg[idx] = out;
+  }
+}
+
+__global__ void __launch_bounds__(256)
+rd_dense_kernel(const float* __restrict__ R, const long long* __restrict__ node_ptr,
+                const long long* __restrict__ sq_ptr, long long total, int nmax, float fill,
+                float* __restrict__ out, unsigned char* __restrict__ mask) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= total) return;
+  const int j = (int)(idx % nmax);
+  const int i = (int)((idx / nmax) % nmax);
+  const long long g = idx / ((long long)nmax * nmax);
+  const int n = (int)(node_ptr[g + 1] - node_ptr[g]);
+  const bool ok = i < n && j < n;
+  out[idx] = ok ? R[sq_ptr[g] + (size_t)i * n + j] : fill;
+  mask[idx] = ok ? 1 : 0;
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256)
 pad_rows_kernel(const T* __restrict__ src, const long long* __restrict__ ptr, long long total,
@@ -300,6 +435,38 @@ extern "C" int pgh_spd_dense_i64(const uint8_t* D, const int64_t* node_ptr, cons
       D, (const long long*)node_ptr, (const long long*)sq_ptr, total, (int)nmax, clamp,
       (long long)fill, (long long*)out, mask);
   return check_launch("spd_dense");
+}
+
+extern "C" int pgh_resistance_f32(const int64_t* edge_src, const int64_t* edge_dst,
+                                  const int64_t* node_ptr, const int64_t* edge_ptr,
+                                  const int64_t* sq_ptr, int64_t n_graphs, int64_t max_nodes,
+                                  float* R, void* stream) {
+  if (n_graphs == 0) return 0;
+  if (!node_ptr || !edge_ptr || !sq_ptr || !R) return arg_error("resistance: null pointer");
+  if (n_graphs < 0 || max_nodes < 1 || max_nodes > kRdMaxNodes)
+    return arg_error("resistance: graphs of 1..128 nodes are supported");
+  const size_t smem = rd_smem_bytes((int)max_nodes);
+  static size_t configured = 48 * 1024;
+  if (smem > configured) {
+    PGH_CUDA(cudaFuncSetAttribute(resistance_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)smem));
+    configured = smem;
+  }
+  resistance_kernel<<<(unsigned)n_graphs, kRdThreads, smem, as_stream(stream)>>>(
+      (const long long*)edge_src, (const long long*)edge_dst, (const long long*)node_ptr,
+      (const long long*)edge_ptr, (const long long*)sq_ptr, (int)max_nodes, R);
+  return check_launch("resistance");
+}
+
+extern "C" int pgh_rd_dense_f32(const float* R, const int64_t* node_ptr, const int64_t* sq_ptr,
+                                int64_t n_graphs, int64_t nmax, float fill, float* out,
+                                uint8_t* mask, void* stream) {
+  const int64_t total = n_graphs * nmax * nmax;
+  if (total == 0) return 0;
+  if (!R || !node_ptr || !sq_ptr || !out || !mask) return arg_error("rd_dense: null pointer");
+  rd_dense_kernel<<<blocks_for(total, 256), 256, 0, as_stream(stream)>>>(
+      R, (const long long*)node_ptr, (const long long*)sq_ptr, total, (int)nmax, fill, out, mask);
+  return check_launch("rd_dense");
 }
 
 extern "C" int pgh_pad_rows(const void* src, const int64_t* ptr, int64_t n_graphs, int64_t nmax,

@@ -267,9 +267,10 @@ def ma_datadict(hb: HostBatch, device, max_dist: int = 5, tuples: str = "khop",
     The host batch is copied in its sparse form and padded ON THE DEVICE (pad / scatter
     kernels of ``hodata.cu``).  ``tuples="khop"``: X holds ``min(dist, max_dist) + 1`` on the
     sampled k-hop tuples and 0 elsewhere; ``tuples="spd"``: X is the shortest-path-distance
-    matrix clamped to ``max_dist + 1``, computed on the device (``spdsampler``)."""
+    matrix clamped to ``max_dist + 1``, computed on the device (``spdsampler``);
+    ``tuples="rd"``: X is the float32 resistance-distance matrix (``rdsampler``)."""
     from .MaData import to_dense_adj, to_dense_x
-    from .MaTupleSampler import spdsampler
+    from .MaTupleSampler import rdsampler, spdsampler
     B = hb.num_graphs
     n = int(np.diff(hb.node_ptr).max())
     node_ptr = _h2d(hb.node_ptr, device, pinned)
@@ -281,6 +282,8 @@ def ma_datadict(hb: HostBatch, device, max_dist: int = 5, tuples: str = "khop",
     m2 = x.mask.unsqueeze(2) & x.mask.unsqueeze(1)
     if tuples == "spd":
         X = spdsampler(ei, hb.node_ptr, max_dist, n)
+    elif tuples == "rd":
+        X = rdsampler(ei, hb.node_ptr, n)
     else:
         tid = _h2d(hb.tupleid, device, pinned)
         feat = torch.clamp(_h2d(hb.tuplefeat, device, pinned), max=max_dist) + 1
