@@ -3,6 +3,11 @@ with pygho_b200: host batches -> ``DevicePrefetcher`` (worker thread + side stre
 steps, or, with ``--resident``, one CUDA-graph replay per step on device-resident batches.
 
     python examples/train_zinc.py --steps 50 [--resident] [--conv SSWL|NGNN|DSSGNN] [--batch 1024]
+                                  [--eval-batches K --eval-every 10]
+
+``--eval-batches K`` holds out K more batches (seeds distinct from the training batches) and every
+``--eval-every`` steps prints their MAE, predicted by graph replay (``static.StaticPredictor``: eval
+mode, no autograd, one-pass BatchNorm blocks), and the evaluation rate.
 """
 from __future__ import annotations
 
@@ -15,6 +20,7 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from examples.zinc_models import SpModel  # noqa: E402
+from pygho_b200 import static as ST  # noqa: E402
 from pygho_b200.dist import FlatGradBucket  # noqa: E402
 from pygho_b200.graph import StepGraph  # noqa: E402
 from pygho_b200.hodata.device import (DeferredScalar, DevicePrefetcher, attach_host_plans,  # noqa: E402
@@ -32,6 +38,8 @@ def main():
     ap.add_argument("--layers", type=int, default=6)
     ap.add_argument("--num-batches", type=int, default=4)
     ap.add_argument("--resident", action="store_true", help="batches stay in HBM, steps replay CUDA graphs")
+    ap.add_argument("--eval-batches", type=int, default=0, help="held-out batches evaluated during training")
+    ap.add_argument("--eval-every", type=int, default=10)
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     torch.backends.cuda.matmul.allow_tf32 = True          # like the reference (zinc.py:30)
@@ -61,6 +69,21 @@ def main():
         attach_host_plans(hb, dd, keys)
         prefetch_plans(dd, keys, embeddings=tables)
         dds.append(dd)
+    evaluate = None
+    if args.eval_batches:
+        eval_hbs = [make_batch(args.batch, seed=100000 + i) for i in range(args.eval_batches)]
+        for hb in eval_hbs:
+            attach_host_plans(hb, sp_datadict(hb, dev, keys), keys)
+        eval_y = torch.cat([torch.from_numpy(hb.y) for hb in eval_hbs]).to(dev).float().unsqueeze(-1)
+        predictor = ST.StaticPredictor(eval_hbs, ST.capacities(eval_hbs, keys), dev, keys, model)
+
+        def evaluate(step):
+            torch.cuda.synchronize()
+            t = time.perf_counter()
+            mae = float((predictor() - eval_y).abs().mean())
+            rate = len(eval_y) / (time.perf_counter() - t)
+            print(f"step {step:4d} validation MAE {mae:.6f} ({len(eval_y)} graphs, {rate:.0f} graphs/s)")
+            return mae
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     if args.resident:
@@ -71,6 +94,8 @@ def main():
             loss = graphs[i % len(graphs)].replay()
             if i % 10 == 0:
                 print(f"step {i:4d} loss {float(loss):.4f}")
+            if evaluate and (i + 1) % args.eval_every == 0:
+                evaluate(i)
     else:
         feeder = DevicePrefetcher(hbs, dev, keys, embeddings=tables)
         reader = DeferredScalar()
@@ -81,11 +106,23 @@ def main():
             if prev is not None and (i - 1) % 10 == 0:
                 print(f"step {i - 1:4d} loss {prev:.4f}")
             feeder.advance()                    # H2D + plans of the next batch, side stream
+            if evaluate and (i + 1) % args.eval_every == 0:
+                evaluate(i)
         print(f"step {args.steps - 1:4d} loss {reader.flush():.4f}")
         feeder.close()
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
-    print(f"{args.steps} steps in {dt:.2f} s = {args.batch * args.steps / dt:.0f} graphs/s")
+    print(f"{args.steps} steps in {dt:.2f} s = {args.batch * args.steps / dt:.0f} graphs/s"
+          + (" (incl. evaluation)" if evaluate else ""))
+    if evaluate:
+        mae = evaluate(args.steps - 1)
+        model.eval()                            # the same batches, eager and unpadded
+        with torch.no_grad():
+            pred = torch.cat([model(sp_datadict(hb, dev, keys)) for hb in eval_hbs])
+        model.train()
+        eager = float((pred - eval_y).abs().mean())
+        print(f"eager no-grad evaluation MAE {eager:.6f} (|replay - eager| = {abs(mae - eager):.1e})")
+        predictor.close()
 
 
 if __name__ == "__main__":

@@ -306,6 +306,16 @@ int pgh_linear_stats_f32(const float* x, int64_t M, int64_t K, const float* w, i
                          float momentum, float* mean, float* rstd, float* running_mean,
                          float* running_var, float* local_out, int64_t* num_batches_tracked,
                          void* ws, size_t ws_bytes, int32_t* tickets, void* stream);
+/* Eval-mode Linear -> BatchNorm1d (running statistics) -> activation in ONE pass (the same
+ * TMA / tcgen05 TF32 GEMM, csrc/linear_stats.cu):
+ *   z = act((x @ w^T + bias - running_mean) * rsqrt(running_var + eps) * gamma + beta) (+ residual)
+ * act: 0 none, 1 SiLU, 2 ReLU.  bias, gamma (1), beta (0), residual ((M, N), 16-byte aligned) and
+ * rows_dev may be NULL; rows >= *rows_dev get z = 0.  Reads the running statistics, writes only z
+ * (32-byte aligned).  Shapes as pgh_linear_stats_supported(); no workspace, no tickets. */
+int pgh_linear_bn_eval_f32(const float* x, int64_t M, int64_t K, const float* w, int64_t N,
+                           const float* bias, const float* gamma, const float* beta,
+                           const float* running_mean, const float* running_var, float eps, int act,
+                           const float* residual, const int32_t* rows_dev, float* z, void* stream);
 /* AdamW (torch.optim.AdamW semantics: decoupled decay, bias correction) over ONE flat buffer of
  * all parameters / gradients / moments of the model (the optimisation step of example/zinc.py:
  * 368-383 as a single launch instead of one multi-tensor launch per dtype/device group).

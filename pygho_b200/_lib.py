@@ -74,6 +74,7 @@ SIGNATURES = {
     "pgh_linear_stats_ws_bytes": (_sz, [_i64]),
     "pgh_linear_stats_f32": (_i, [_p, _i64, _i64, _p, _i64, _p, _p, _p, _f, _f, _p, _p, _p, _p, _p, _p,
                                   _p, _sz, _p, _p]),
+    "pgh_linear_bn_eval_f32": (_i, [_p, _i64, _i64, _p, _i64, _p, _p, _p, _p, _p, _f, _i, _p, _p, _p, _p]),
     "pgh_bn_sync_finalize_f32": (_i, [_p, _i64, _i64, _f, _f, _p, _p, _p, _p, _p, _p]),
     "pgh_bn_act_res_fwd_f32": (_i, [_p, _p, _p, _p, _p, _i64, _i64, _p, _i, _p, _p, _p]),
     "pgh_bn_act_bwd_reduce_f32": (_i, [_p, _p, _p, _p, _p, _p, _i64, _i64, _p, _i, _p, _p, _p, _i,

@@ -77,6 +77,15 @@ __device__ __forceinline__ void pdl_enter() {
 #endif
   asm volatile("griddepcontrol.wait;" ::: "memory");
 }
+
+// activation of the MLP blocks (0 none, 1 SiLU, 2 ReLU); one definition so that the BatchNorm
+// apply pass (fused_mlp.cu) and the eval GEMM epilogue (linear_stats.cu) round identically
+template <int ACT>
+__device__ __forceinline__ float act_fwd(float x) {
+  if (ACT == 1) return x / (1.f + __expf(-x));
+  if (ACT == 2) return fmaxf(x, 0.f);
+  return x;
+}
 #endif
 
 }  // namespace pgh

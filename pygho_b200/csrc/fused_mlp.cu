@@ -85,13 +85,6 @@ __device__ __forceinline__ long long valid_rows(long long rows, const int* __res
 }
 
 template <int ACT>
-__device__ __forceinline__ float act_fwd(float x) {
-  if (ACT == 1) return x / (1.f + __expf(-x));
-  if (ACT == 2) return fmaxf(x, 0.f);
-  return x;
-}
-
-template <int ACT>
 __device__ __forceinline__ float act_grad(float x) {
   if (ACT == 1) {
     const float s = 1.f / (1.f + __expf(-x));

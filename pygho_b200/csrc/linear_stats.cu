@@ -18,6 +18,12 @@
 //   end      per-CTA partials -> two-level ticketed combine (ticket.cuh) -> mean / rstd /
 //            running statistics (or the rank-local triple for SyncBN) by the last CTA
 //
+// Eval mode (kEval, pgh_linear_bn_eval_f32): the same producer, MMA issuer and TMEM double
+// buffer; the BatchNorm uses its running statistics, so the whole block is one epilogue
+//   z[r, c] = act(acc[r, c] * s[c] + t[c]) (+ residual[r, c]),
+//   s = gamma * rsqrt(running_var + eps),  t = (bias - running_mean) * s + beta
+// with no statistics, no workspace and no combine.  Rows >= rows_dev get 0 (as bn_act_fwd).
+//
 // TF32 like the reference on a GPU (example/zinc.py:30 set_float32_matmul_precision('high')).
 // HBM-bound by design: per 128-row tile 128 x K x 4 B in, 64 KB out; W stays in L2.
 // Shapes: N in {128, 256, 384}, K % 32 == 0 (every large Linear of the SSWL+/NGNN/DSSGNN/PPGN/I2
@@ -166,7 +172,16 @@ struct LsBars {
   unsigned long long full[kLsMaxStages], empty[kLsMaxStages], tfull[2], tempty[2];
 };
 
-template <int NT>
+// eval-mode operands (unused by the training instantiation)
+struct LsEvalArgs {
+  const float* gamma;        // NULL: 1
+  const float* beta;         // NULL: 0
+  const float* residual;     // NULL: none; else (M, N) row-major, 16-byte aligned
+};
+
+// kEval = false: Linear + BatchNorm statistics (training); kEval = true: Linear + BatchNorm with
+// running statistics + activation ACT (+ residual) written to y
+template <int NT, bool kEval, int ACT>
 __global__ void __launch_bounds__(kLsThreads, 1)
 linear_stats_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w,
                     const float* __restrict__ bias, long long M, int K, const int* __restrict__ rows_dev,
@@ -174,7 +189,7 @@ linear_stats_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_cons
                     int grp, int ngroups, int* __restrict__ tickets, float eps, float momentum,
                     float* __restrict__ mean, float* __restrict__ rstd, float* __restrict__ running_mean,
                     float* __restrict__ running_var, float* __restrict__ local_out,
-                    long long* __restrict__ nbt) {
+                    long long* __restrict__ nbt, const LsEvalArgs ev) {
   extern __shared__ unsigned char ls_smem_raw[];
   __shared__ LsBars bars;
   __shared__ uint32_t tmem_holder;
@@ -272,7 +287,56 @@ linear_stats_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_cons
         ls_umma_commit(ls_smem_u32(&bars.tfull[buf]));               // accumulator complete
       }
     }
-  } else if (warp >= 4) {
+  } else if (kEval && warp >= 4) {
+    // ===== eval epilogue: TMEM -> scale / shift -> activation (+ residual) -> global =====
+    const int q = warp - 4;
+    float* s_scale = s_part[0][0];                // the statistics scratch is free in eval mode
+    float* s_shift = s_part[0][1];
+    // running statistics / parameters are written by earlier kernels (optimizer, load_state_dict
+    // copies): read after griddepcontrol.wait
+    for (int c = threadIdx.x - 128; c < kLsBN; c += 128) {
+      const float sc = (ev.gamma ? __ldg(ev.gamma + c) : 1.f) * rsqrtf(__ldg(running_var + c) + eps);
+      s_scale[c] = sc;
+      s_shift[c] = fmaf((bias ? __ldg(bias + c) : 0.f) - __ldg(running_mean + c), sc,
+                        ev.beta ? __ldg(ev.beta + c) : 0.f);
+    }
+    asm volatile("bar.sync 1, 128;" ::: "memory");   // the four epilogue warps only
+    int it = 0;
+    for (int tile = blockIdx.x; tile < m_tiles; tile += gridDim.x, ++it) {
+      const int buf = kBufs == 2 ? (it & 1) : 0;
+      const uint32_t aphase = (uint32_t)(kBufs == 2 ? (it >> 1) : it) & 1u;
+      ls_mbar_wait(ls_smem_u32(&bars.tfull[buf]), aphase);
+      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      const long long row = (long long)tile * kLsBM + q * 32 + lane;
+      const bool row_ok = row < M, row_valid = row < rows_valid;
+      float* yrow = y + (size_t)row * kLsBN;
+      const float4* rrow =
+          ev.residual ? reinterpret_cast<const float4*>(ev.residual + (size_t)row * kLsBN) : nullptr;
+#pragma unroll
+      for (int cb = 0; cb < 4 * NT; ++cb) {
+        float v[32];
+        ls_tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * kLsBN + cb * 32), v);
+        if (row_ok) {
+          float o[32];
+#pragma unroll
+          for (int i = 0; i < 32; ++i)
+            o[i] = row_valid ? act_fwd<ACT>(fmaf(v[i], s_scale[cb * 32 + i], s_shift[cb * 32 + i])) : 0.f;
+          if (ev.residual && row_valid) {
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              const float4 r = __ldg(rrow + cb * 8 + i);
+              o[4 * i] += r.x; o[4 * i + 1] += r.y; o[4 * i + 2] += r.z; o[4 * i + 3] += r.w;
+            }
+          }
+#pragma unroll
+          for (int i = 0; i < 32; i += 8) ls_st_global_v8(yrow + cb * 32 + i, o + i);
+        }
+      }
+      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      __syncwarp();
+      if (lane == 0) ls_mbar_arrive(ls_smem_u32(&bars.tempty[buf]));
+    }
+  } else if (!kEval && warp >= 4) {
     // ===== epilogue: TMEM -> registers -> global, column statistics =====
     const int q = warp - 4;                       // TMEM lane quarter this warp may access
     double acc_s[4 * NT], acc_q[4 * NT];
@@ -325,15 +389,17 @@ linear_stats_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_cons
   if (warp == 2)
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kLsTmemCols)
                  : "memory");
-  for (int t = threadIdx.x; t < 2 * kLsBN; t += kLsThreads) {
-    const int which = t / kLsBN, c = t - which * kLsBN;
-    const float tot = ((s_part[0][which][c] + s_part[1][which][c]) + s_part[2][which][c]) + s_part[3][which][c];
-    part[(size_t)blockIdx.x * 2 * kLsBN + t] = tot;
+  if constexpr (!kEval) {
+    for (int t = threadIdx.x; t < 2 * kLsBN; t += kLsThreads) {
+      const int which = t / kLsBN, c = t - which * kLsBN;
+      const float tot = ((s_part[0][which][c] + s_part[1][which][c]) + s_part[2][which][c]) + s_part[3][which][c];
+      part[(size_t)blockIdx.x * 2 * kLsBN + t] = tot;
+    }
+    if (!ticketed_combine(part, part2, 2 * kLsBN, gridDim.x, grp, ngroups, tickets, s_fin)) return;
+    // statistics of (y - bias): shift = bias
+    bn_finalize_stats(s_fin, kLsBN, (double)rows_valid, bias, eps, momentum, mean, rstd, running_mean,
+                      running_var, local_out, nbt);
   }
-  if (!ticketed_combine(part, part2, 2 * kLsBN, gridDim.x, grp, ngroups, tickets, s_fin)) return;
-  // statistics of (y - bias): shift = bias
-  bn_finalize_stats(s_fin, kLsBN, (double)rows_valid, bias, eps, momentum, mean, rstd, running_mean,
-                    running_var, local_out, nbt);
 }
 
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -398,26 +464,30 @@ extern "C" size_t pgh_linear_stats_ws_bytes(int64_t M) {
          (size_t)g.ngroups * 2 * kMaxN * sizeof(float) + 256;
 }
 
-template <int NT>
+template <int NT, bool kEval, int ACT>
 static int ls_launch(const CUtensorMap& map_x, const CUtensorMap& map_w, const float* bias, int64_t M,
                      int64_t K, const int32_t* rows_dev, float* y, const LsGeom& g, void* ws,
                      int32_t* tickets, float eps, float momentum, float* mean, float* rstd,
                      float* running_mean, float* running_var, float* local_out, int64_t* nbt,
-                     cudaStream_t s) {
+                     const LsEvalArgs& ev, cudaStream_t s) {
   using Cfg = LsCfg<NT>;
   static bool attr_set = false;
   if (!attr_set) {
-    PGH_CUDA(cudaFuncSetAttribute(linear_stats_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)Cfg::kSmemBytes));
+    PGH_CUDA(cudaFuncSetAttribute(linear_stats_kernel<NT, kEval, ACT>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
     attr_set = true;
   }
-  float* part = reinterpret_cast<float*>(ws);
-  float* part2 = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) +
-                                          ((size_t)g.grid * 2 * Cfg::N * sizeof(float) + 255) / 256 * 256);
-  launch_pdl(linear_stats_kernel<NT>, dim3(g.grid), dim3(kLsThreads), Cfg::kSmemBytes, s,
+  float* part = nullptr;
+  float* part2 = nullptr;
+  if (!kEval) {
+    part = reinterpret_cast<float*>(ws);
+    part2 = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) +
+                                     ((size_t)g.grid * 2 * Cfg::N * sizeof(float) + 255) / 256 * 256);
+  }
+  launch_pdl(linear_stats_kernel<NT, kEval, ACT>, dim3(g.grid), dim3(kLsThreads), Cfg::kSmemBytes, s,
       map_x, map_w, bias, M, (int)K, rows_dev, y, part, part2, g.grp, g.ngroups, tickets, eps, momentum,
-      mean, rstd, running_mean, running_var, local_out, reinterpret_cast<long long*>(nbt));
-  return check_launch("linear_stats");
+      mean, rstd, running_mean, running_var, local_out, reinterpret_cast<long long*>(nbt), ev);
+  return check_launch(kEval ? "linear_bn_eval" : "linear_stats");
 }
 
 extern "C" int pgh_linear_stats_f32(const float* x, int64_t M, int64_t K, const float* w, int64_t N,
@@ -437,10 +507,42 @@ extern "C" int pgh_linear_stats_f32(const float* x, int64_t M, int64_t K, const 
     return arg_error("linear_stats: cuTensorMapEncodeTiled failed");
   const LsGeom g = ls_geom(M);
   cudaStream_t s = as_stream(stream);
-#define PGH_LS(NT_) ls_launch<NT_>(map_x, map_w, bias, M, K, rows_dev, y, g, ws, tickets, eps, momentum, \
-                                   mean, rstd, running_mean, running_var, local_out, num_batches_tracked, s)
+#define PGH_LS(NT_) ls_launch<NT_, false, 0>(map_x, map_w, bias, M, K, rows_dev, y, g, ws, tickets, eps, \
+                                   momentum, mean, rstd, running_mean, running_var, local_out,          \
+                                   num_batches_tracked, LsEvalArgs{}, s)
   if (N == 128) return PGH_LS(1);
   if (N == 256) return PGH_LS(2);
   return PGH_LS(3);
 #undef PGH_LS
+}
+
+extern "C" int pgh_linear_bn_eval_f32(const float* x, int64_t M, int64_t K, const float* w, int64_t N,
+                                      const float* bias, const float* gamma, const float* beta,
+                                      const float* running_mean, const float* running_var, float eps,
+                                      int act, const float* residual, const int32_t* rows_dev, float* z,
+                                      void* stream) {
+  if (!x || !w || !running_mean || !running_var || !z) return arg_error("linear_bn_eval: null pointer");
+  if (!pgh_linear_stats_supported(M, K, N))
+    return arg_error("linear_bn_eval: need N in {128, 256, 384}, K % 32 == 0, K <= 4096");
+  if (act < 0 || act > 2) return arg_error("linear_bn_eval: act");
+  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(w) |
+       reinterpret_cast<uintptr_t>(residual)) & 15)
+    return arg_error("linear_bn_eval: x, w and residual must be 16-byte aligned");
+  if (reinterpret_cast<uintptr_t>(z) & 31) return arg_error("linear_bn_eval: z must be 32-byte aligned");
+  CUtensorMap map_x, map_w;
+  if (!make_map(&map_x, x, M, K) || !make_map(&map_w, w, N, K))
+    return arg_error("linear_bn_eval: cuTensorMapEncodeTiled failed");
+  const LsGeom g = ls_geom(M);
+  const LsEvalArgs ev{gamma, beta, residual};
+  cudaStream_t s = as_stream(stream);
+  float* rm = const_cast<float*>(running_mean);     // read only: the eval kernel writes no statistics
+  float* rv = const_cast<float*>(running_var);
+#define PGH_EV(NT_, A_) ls_launch<NT_, true, A_>(map_x, map_w, bias, M, K, rows_dev, z, g, nullptr, nullptr, \
+                                                 eps, 0.f, nullptr, nullptr, rm, rv, nullptr, nullptr, ev, s)
+#define PGH_EV_ACT(NT_) return act == 1 ? PGH_EV(NT_, 1) : act == 2 ? PGH_EV(NT_, 2) : PGH_EV(NT_, 0)
+  if (N == 128) PGH_EV_ACT(1);
+  if (N == 256) PGH_EV_ACT(2);
+  PGH_EV_ACT(3);
+#undef PGH_EV_ACT
+#undef PGH_EV
 }

@@ -124,9 +124,10 @@ class MLP(nn.Module):
             out = self.lins(x)
             return out if residual is None else out + residual
         # Linear -> BatchNorm(train) -> SiLU/ReLU blocks go through the fused kernels
-        # (pygho_b200/csrc/fused_mlp.cu); anything else runs module by module.
+        # (pygho_b200/csrc/fused_mlp.cu), inference blocks (BatchNorm in eval mode, no autograd)
+        # through ops.linear_bn_eval; anything else runs module by module.
         from .. import static
-        from ..ops import ACT_CODE, LinearBNAct
+        from ..ops import ACT_CODE, LinearBNAct, linear_bn_eval
         mods = list(self.lins)
         shape = x.shape
         h = x.reshape(-1, shape[-1])
@@ -145,6 +146,15 @@ class MLP(nn.Module):
                                       getattr(bn, "_pgh_sync_group", None),
                                       bn.num_batches_tracked if bn.track_running_stats else None)
                 i += 3
+                continue
+            blk = _match_eval_block(mods, i)
+            if blk is not None:
+                bn, act, n = blk
+                res = None
+                if residual is not None and i + n == len(mods):
+                    res, residual = residual.reshape(-1, residual.shape[-1]), None
+                h = linear_bn_eval(h, m.weight, m.bias, bn, act, res, static.rows_dev_for(h.shape[0]))
+                i += n
             else:
                 h = m(h)
                 i += 1
@@ -164,8 +174,29 @@ def _match_block(mods, i):
     return bn, act
 
 
+def _match_eval_block(mods, i):
+    """(BatchNorm1d, act name, block length) if mods[i:] starts with Linear, BatchNorm(eval, running
+    statistics), [Dropout(eval)], SiLU/ReLU and autograd is off: an inference block that needs no
+    backward, so the BatchNorm folds into the GEMM epilogue.  With gradients enabled (e.g. fine-
+    tuning with a frozen BatchNorm) the block stays on the stock modules."""
+    import torch
+    if torch.is_grad_enabled() or i + 2 >= len(mods) or not isinstance(mods[i], nn.Linear) \
+            or type(mods[i + 1]) is not BatchNorm:
+        return None
+    bn = mods[i + 1].norm
+    j = i + 2
+    if isinstance(mods[j], nn.Dropout) and not mods[j].training and j + 1 < len(mods):
+        j += 1
+    act = {nn.SiLU: "silu", nn.ReLU: "relu"}.get(type(mods[j]))
+    if act is None or bn.training or not bn.track_running_stats or bn.running_mean is None \
+            or bn.num_features % 4 or bn.num_features > 1024:
+        return None
+    return bn, act, j + 1 - i
+
+
 def _fusable(lins, x: Tensor) -> bool:
     import torch
     return (isinstance(lins, nn.Sequential) and x.is_cuda and x.dtype == torch.float32
             and x.numel() > 0 and torch.is_grad_enabled() is not None
-            and any(_match_block(list(lins), i) is not None for i in range(len(lins))))
+            and any(_match_block(list(lins), i) is not None or _match_eval_block(list(lins), i)
+                    is not None for i in range(len(lins))))

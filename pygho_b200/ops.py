@@ -501,6 +501,42 @@ def _linear_stats_fake(x, weight, bias, eps, momentum, running_mean, running_var
     return y, x.new_empty((N,)), x.new_empty((N,))
 
 
+_LIB.define("linear_bn_eval(Tensor x, Tensor weight, Tensor? bias, Tensor? gamma, Tensor? beta, "
+            "Tensor running_mean, Tensor running_var, float eps, int act, Tensor? residual=None, "
+            "Tensor? rows_dev=None) -> Tensor")
+
+
+def _linear_bn_eval_cuda(x, weight, bias, gamma, beta, running_mean, running_var, eps, act,
+                         residual=None, rows_dev=None):
+    """z = act(BatchNorm_eval(x @ W^T + b)) (+ residual) in one pass (csrc/linear_stats.cu)."""
+    x, weight, bias, residual = _f32c(x), _f32c(weight), _f32c(bias), _f32c(residual)
+    if x.ndim != 2 or weight.ndim != 2 or weight.shape[1] != x.shape[1]:
+        raise ValueError("linear_bn_eval: need x (M, K) and weight (N, K)")
+    M, K = x.shape
+    N = weight.shape[0]
+    for name, v in (("bias", bias), ("gamma", gamma), ("beta", beta),
+                    ("running_mean", running_mean), ("running_var", running_var)):
+        if v is not None and v.numel() != N:
+            raise ValueError(f"linear_bn_eval: {name} must have {N} elements")
+    if residual is not None and residual.shape != (M, N):
+        raise ValueError("linear_bn_eval: residual must have the shape of the output")
+    z = torch.empty((M, N), dtype=torch.float32, device=x.device)
+    call("pgh_linear_bn_eval_f32", ptr(x), M, K, ptr(weight), N, ptr(bias), ptr(_f32c(gamma)),
+         ptr(_f32c(beta)), ptr(_f32c(running_mean)), ptr(_f32c(running_var)), float(eps), int(act),
+         ptr(residual), ptr(_rows_dev(rows_dev)), ptr(z), stream_ptr(x.device))
+    _lib.count_launch()
+    return z
+
+
+_LIB.impl("linear_bn_eval", _linear_bn_eval_cuda, "CUDA")
+
+
+@torch.library.register_fake("pygho_b200::linear_bn_eval")
+def _linear_bn_eval_fake(x, weight, bias, gamma, beta, running_mean, running_var, eps, act,
+                         residual=None, rows_dev=None):
+    return x.new_empty((x.shape[0], weight.shape[0]))
+
+
 _LIB.define("bn_stats_local(Tensor y, Tensor? rows_dev=None, "
             "Tensor(a!)? num_batches_tracked=None) -> Tensor")
 
@@ -1229,3 +1265,41 @@ class LinearBNAct(torch.autograd.Function):
                 None, None, None, None, None,
                 dz if (len(need) > 10 and need[10]) else None,   # residual: gradient passes through
                 None, None, None)
+
+
+# Output widths N at which the one-pass eval kernel beats cuBLAS + the bn_act_fwd pass: none on a
+# B200 (1000 W).  At 230 147 rows with SiLU it takes 221 / 210 / 512 / 877 us for 384->128,
+# 128->128, 384->256 and 384->384 against 132 / 98 / 201 / 308 us for the fallback
+# (profiles/eval_times.txt, DESIGN.md section 4.6): the four epilogue warps, one per SM
+# sub-partition, are issue-bound on scale / shift / SiLU / stores, and N > 128 re-reads W per tile.
+_EVAL_GEMM_WIDTHS: tuple = ()
+
+
+def linear_bn_eval_ok(x: Tensor, weight: Tensor) -> bool:
+    """Whether :func:`linear_bn_eval` runs the one-pass TF32 kernel for this shape: TF32 allowed
+    (as for :func:`linear_stats_ok`), enough rows, a supported shape and a width where the
+    kernel was measured faster than the fallback."""
+    return (torch.backends.cuda.matmul.allow_tf32 and x.dtype == torch.float32 and x.ndim == 2
+            and x.is_cuda and weight.dtype == torch.float32 and x.shape[0] >= _FUSED_GEMM_MIN_ROWS
+            and weight.shape[0] in _EVAL_GEMM_WIDTHS
+            and bool(_lib.load().pgh_linear_stats_supported(x.shape[0], x.shape[1], weight.shape[0])))
+
+
+def linear_bn_eval(x: Tensor, weight: Tensor, bias: Optional[Tensor], bn: torch.nn.BatchNorm1d,
+                   act: str, residual: Optional[Tensor] = None,
+                   rows_dev: Optional[Tensor] = None) -> Tensor:
+    """Inference of a Linear -> BatchNorm1d (eval: running statistics) -> ``act`` block on 2-D
+    ``x``, plus ``residual``: ``act((x W^T + b - running_mean) / sqrt(running_var + eps) * gamma
+    + beta) (+ residual)``.  Rows >= ``rows_dev`` (capacity-padded batches) are 0.  Not
+    differentiable, and never writes the BatchNorm's running statistics.
+
+    One pass through the TMA / tcgen05 GEMM with the BatchNorm in its epilogue
+    (csrc/linear_stats.cu) where :func:`linear_bn_eval_ok`; otherwise ``F.linear`` followed by the
+    fused BatchNorm-apply kernel with ``mean = running_mean``, ``rstd = rsqrt(running_var + eps)``."""
+    code = ACT_CODE[act]
+    if linear_bn_eval_ok(x, weight):
+        return _ops.linear_bn_eval(x, weight, bias, bn.weight, bn.bias, bn.running_mean,
+                                   bn.running_var, bn.eps, code, residual, rows_dev)
+    y = torch.nn.functional.linear(x, weight, bias)
+    rstd = torch.rsqrt(bn.running_var + bn.eps)
+    return _ops.bn_act_fwd(y, bn.running_mean, rstd, bn.weight, bn.bias, code, residual, rows_dev)

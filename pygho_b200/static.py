@@ -93,13 +93,19 @@ def capacities(host_batches: Iterable[HostBatch], keys: Sequence[str], margin: f
     return caps
 
 
-def pad_host_batch(hb: HostBatch, caps: dict, keys: Sequence[str]) -> HostBatch:
-    """Pad a collated batch (with its host plans) to ``caps``; see the module docstring."""
+def pad_host_batch(hb: HostBatch, caps: dict, keys: Sequence[str],
+                   fewer_graphs: bool = False) -> HostBatch:
+    """Pad a collated batch (with its host plans) to ``caps``; see the module docstring.
+
+    ``fewer_graphs``: accept a batch of ``B < caps["B"]`` graphs; graphs ``B .. caps["B"] - 1``
+    are then empty and the dummy graph is ``caps["B"]``.  For evaluation only (the graph rows
+    are read back as ``[:B]``): a training loss over ``num_valid_graphs`` would count the empty
+    graphs."""
     if hb.tupleid.shape[0] != 2:
         raise NotImplementedError("static batches support 2-D tuples")
     N, nA, nX, B = hb.num_nodes, hb.edge_index.shape[1], hb.tupleid.shape[1], hb.num_graphs
-    Nc, Ac, Xc = caps["N"], caps["A"], caps["X"]
-    if B != caps["B"] or N >= Nc or nA >= Ac or nX >= Xc:
+    Nc, Ac, Xc, Bc = caps["N"], caps["A"], caps["X"], caps["B"]
+    if not (B == Bc or (fewer_graphs and B < Bc)) or N >= Nc or nA >= Ac or nX >= Xc:
         raise ValueError("batch does not fit the capacities (every array needs >= 1 pad row)")
 
     def pad1(a, n, value):
@@ -128,10 +134,10 @@ def pad_host_batch(hb: HostBatch, caps: dict, keys: Sequence[str]) -> HostBatch:
         out[2, T:] = n_rows[ops[1]][1]
         plans[key] = out
     padded = replace(
-        hb, num_graphs=B + 1, num_nodes=Nc,
+        hb, num_graphs=Bc + 1, num_nodes=Nc,
         x=pad1(hb.x, Nc, 0), edge_index=pad2(hb.edge_index, Ac, Nc - 1),
         edge_attr=pad1(hb.edge_attr, Ac, 0), tupleid=pad2(hb.tupleid, Xc, Nc - 1),
-        tuplefeat=pad1(hb.tuplefeat, Xc, 0), batch=pad1(hb.batch, Nc, B), y=pad1(hb.y, B + 1, 0.0),
+        tuplefeat=pad1(hb.tuplefeat, Xc, 0), batch=pad1(hb.batch, Nc, Bc), y=pad1(hb.y, Bc + 1, 0.0),
         plans=plans)
     padded.valid = np.array([nX, N, B], dtype=np.int32)
     return padded
@@ -347,7 +353,8 @@ class StaticFeeder:
     worker thread loads the next host batch into the other slot on a side stream.
 
     ``host_batches``: padded :class:`HostBatch` objects (:func:`pad_host_batch`), cycled.
-    ``step_fn(dd)`` must be capturable (see pygho_b200/graph.py) and return the loss tensor."""
+    ``step_fn(dd)`` must be capturable (see pygho_b200/graph.py) and return the step's output
+    tensor (e.g. the loss)."""
 
     def __init__(self, host_batches, caps, device, keys, step_fn, pinned: Optional[dict] = None,
                  threaded: bool = True):
@@ -426,8 +433,8 @@ class StaticFeeder:
             self._done[index & 1].set()
 
     def step(self) -> torch.Tensor:
-        """Replay the training step on the current batch; returns the (static) loss tensor of
-        the slot -- read it (or copy it) before the same slot is replayed two steps later."""
+        """Replay the step on the current batch; returns the (static) output tensor of the
+        slot -- read it (or copy it) before the same slot is replayed two steps later."""
         slot = self.pos & 1
         self._done[slot].wait()
         if self._error is not None:
@@ -447,3 +454,50 @@ class StaticFeeder:
             self._worker.join(timeout=10)
             self._jobs = None
         self.graphs = []
+
+
+class StaticPredictor:
+    """Graph-replayed evaluation of a fixed held-out set: ``predictor()`` returns the model's
+    predictions for every graph of ``host_batches``, in order, as one ``(sum B_i, out)`` device
+    tensor.  Built on :class:`StaticFeeder` (same scope: sparse mode, 2-D tuples).
+
+    ``host_batches``: UNPADDED :class:`HostBatch` objects with their host plans; they are padded
+    here to ``caps`` (:func:`capacities` over these batches), and may hold fewer graphs than
+    ``caps["B"]``.  ``model(dd)`` is captured on the two slots in ``eval()`` mode under
+    ``torch.no_grad()`` -- the BatchNorm blocks take the one-pass inference path
+    (ops.linear_bn_eval) and nothing writes the running statistics -- and the model's training
+    flag is restored afterwards.  ``no_grad`` rather than ``inference_mode``: the plans are cached
+    on the datadicts' index tensors, and inference tensors could not be used by a later training
+    step on the same data.
+
+    Lifetime: the graphs read the parameters and running statistics in place, so they follow
+    optimizer steps and ``load_state_dict``; anything that reallocates them (``.to()``,
+    replacing a module or a parameter) needs a new predictor."""
+
+    def __init__(self, host_batches, caps, device, keys, model, pinned: Optional[dict] = None,
+                 threaded: bool = True):
+        hbs = list(host_batches)
+        self.counts = [hb.num_graphs for hb in hbs]
+        padded = [pad_host_batch(hb, caps, keys, fewer_graphs=True) for hb in hbs]
+        was_training = model.training
+        model.eval()
+        try:
+            with torch.no_grad():
+                self.feeder = StaticFeeder(padded, caps, device, keys, model, pinned, threaded)
+        finally:
+            model.train(was_training)
+
+    def __call__(self) -> torch.Tensor:
+        """Replay every batch once; rows ``[:B_i]`` of each replay's output (the dummy pad graph
+        and any empty graphs dropped), concatenated in batch order.  Stream-ordered."""
+        out, off = None, 0
+        for b in self.counts:
+            pred = self.feeder.step()
+            if out is None:
+                out = pred.new_empty((sum(self.counts),) + tuple(pred.shape[1:]))
+            out[off:off + b].copy_(pred[:b])
+            off += b
+        return out
+
+    def close(self):
+        self.feeder.close()
