@@ -39,8 +39,8 @@ const char* pgh_last_error(void);
 int pgh_abi_version(void);
 /* fills {device ordinal, SM count, L2 bytes, cc major, cc minor}; host pointer */
 int pgh_device_info(int32_t* out5);
-/* run-time tuning knobs; host call.  Keys 2..5 = fused BatchNorm kernels (CTAs per SM, rows in
- * flight, reverse walk, forward elements in flight; 0 = default): only the work split changes,
+/* run-time tuning knobs; host call.  Keys 2, 3 and 5 = fused BatchNorm kernels (CTAs per SM, rows
+ * in flight, forward elements in flight; 0 = default): only the work split changes,
  * reductions stay deterministic for a given setting.  Key 7 = bit mask of mamamm profiling
  * ablations (0 = off, the default; others switch parts of the kernel off).  Key 8 = programmatic dependent
  * launch (1 = on, the default; 0 = every kernel fully serialised).  Any other key is an

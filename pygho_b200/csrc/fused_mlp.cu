@@ -38,11 +38,9 @@ namespace pgh {
 constexpr int kBnThreads = 256;
 
 // run-time tuning (pgh_set_tuning): [2] partial-reduction CTAs per SM (default 4), [3] rows in
-// flight per thread in the backward kernels (2 or 4), [4] 1 = the apply passes walk the rows in
-// the opposite direction of the reduce pass before them (the tail of that pass is still in the
-// 126 MB L2), [5] elements in flight per thread of the forward apply (1, 2 or 4; default 2).
-// Sweep on B200 (profiles/r1_bn_sweep.txt): 2 rows in flight and 4 CTAs/SM are best, the
-// reverse walk buys nothing (the L2 does not keep the tail of a streaming pass)
+// flight per thread in the backward kernels (2 or 4), [5] elements in flight per thread of the
+// forward apply (1, 2 or 4; default 2).  Sweep on B200 (profiles/r1_bn_sweep.txt): 2 rows in
+// flight and 4 CTAs/SM are best.
 static int bn_tune(int key, int dflt) { return g_tune[key] > 0 ? g_tune[key] : dflt; }
 
 constexpr int kBnMaxGroups = 63;   // ticket words per launch: 1 + groups <= 64
@@ -170,7 +168,7 @@ __global__ void bn_sync_finalize_kernel(const float* __restrict__ gathered, int 
   const double var = n > 0.0 ? m2 / n : 0.0;
   mean[c] = (float)m;
   rstd[c] = (float)(1.0 / sqrt(var + (double)eps));
-  if (running_mean) {
+  if (running_mean && n > 0.0) {              // no rows on any rank: running statistics unchanged
     const double unbiased = n > 1.0 ? m2 / (n - 1.0) : var;
     running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)m;
     running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;

@@ -664,7 +664,7 @@ static Geometry geometry(int64_t n_rows, int64_t dense, bool aligned) {
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 
-// run-time tuning knobs (pgh_set_tuning): [2..5] fused BN kernels (fused_mlp.cu), [7] mamamm
+// run-time tuning knobs (pgh_set_tuning): [2, 3, 5] fused BN kernels (fused_mlp.cu), [7] mamamm
 // profiling ablations (mamamm_smem.cu), [8] programmatic dependent launch (common.cuh)
 int g_tune[16] = {0, 0, 0, 0, 0, 0, 0, 0, /* [8] */ 1, 0, 0, 0, 0, 0, 0, 0};
 
@@ -783,7 +783,7 @@ extern "C" const char* pgh_last_error(void) { return pgh::g_err; }
 extern "C" int pgh_abi_version(void) { return 4; }
 
 extern "C" int pgh_set_tuning(int key, int value) {
-  if (!((key >= 2 && key <= 5) || key == 7 || key == 8)) return arg_error("set_tuning: key");
+  if (!(key == 2 || key == 3 || key == 5 || key == 7 || key == 8)) return arg_error("set_tuning: key");
   pgh::g_tune[key] = value;
   return 0;
 }

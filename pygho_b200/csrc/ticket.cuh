@@ -100,7 +100,9 @@ __device__ inline bool ticketed_combine(const float* part, float* part2, int W, 
 
 // Per-channel epilogue of a BatchNorm statistics reduction, run by the CTA that won the ticket:
 // fin[c] = sum (y - shift), fin[C + c] = sum (y - shift)^2 over n rows.
-//   local_out == NULL : mean, rstd (+ running statistics with the unbiased variance)
+//   local_out == NULL : mean, rstd (+ running statistics with the unbiased variance; with n == 0
+//                       mean = 0 and rstd = 1/sqrt(eps), and the running statistics keep their
+//                       values: an empty batch is not evidence of mean 0 and variance 0)
 //   local_out != NULL : the rank-local (mean, M2, count) rows for cross-rank merging (SyncBN)
 // shift may be NULL (= 0).  nbt: BatchNorm1d.num_batches_tracked (int64) or NULL.
 __device__ inline void bn_finalize_stats(const double* fin, int C, double n,
@@ -126,7 +128,7 @@ __device__ inline void bn_finalize_stats(const double* fin, int C, double n,
     const double var = n > 0.0 ? m2 / n : 0.0;              // biased variance
     mean[c] = (float)m;
     rstd[c] = (float)(1.0 / sqrt(var + (double)eps));
-    if (running_mean) {
+    if (running_mean && n > 0.0) {
       const double unbiased = n > 1.0 ? m2 / (n - 1.0) : var;
       running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)m;
       running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;

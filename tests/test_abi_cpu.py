@@ -52,8 +52,9 @@ def test_argument_errors_are_reported():
         _lib.call("pgh_seg_gmr_f32", None, None, None, None, None, None, 4, 0, 8, 0, None, None)
     with pytest.raises(_lib.KernelError, match="aggr"):
         _lib.call("pgh_seg_gmr_f32", 16, None, None, None, None, None, 4, 0, 8, 9, 16, None)
-    with pytest.raises(_lib.KernelError, match="set_tuning: key"):
-        _lib.call("pgh_set_tuning", 0, 2)
+    for key in (0, 4):                                   # 4: the retired reverse-walk knob
+        with pytest.raises(_lib.KernelError, match="set_tuning: key"):
+            _lib.call("pgh_set_tuning", key, 2)
 
 
 def test_api_surface_names():
