@@ -228,6 +228,15 @@ masked_pool_warp_kernel(const float4* __restrict__ data, const unsigned char* __
   if (out_mask && ch == 0) out_mask[rest] = cnt > 0;
 }
 
+// max / min backward: the tie count of one channel, or -1 once a valid entry is the infinite
+// extreme (+inf for max, -inf for min).  The forward replaced that inf by 0 (filterinf), and like
+// the reference's masked_fill the replaced output passes no gradient, not even to valid zeros.
+// The -1 is sticky under pool_cnt_add, the combine of partial counts; weights need a count > 0.
+__device__ __forceinline__ int pool_tie(int c, float x, float ov, float pole) {
+  return (c < 0 || x == pole) ? -1 : c + (x == ov);
+}
+__device__ __forceinline__ int pool_cnt_add(int a, int b) { return (a < 0 || b < 0) ? -1 : a + b; }
+
 // Backward, warp-cooperative (dense % 128 == 0): mask bits by ballot, stores never wait for a
 // mask load; the tie / valid counts of mean, max and min come from the same bit sets.
 template <int AGGR, bool SPLIT>
@@ -255,6 +264,7 @@ masked_pool_bwd_warp_kernel(const float4* __restrict__ data, const unsigned char
   const long long pstep = v.inner, dstep = (long long)v.inner * v.c4;
   const float4 g = g_out[rest * v.c4 + ch];
   constexpr bool kExt = (AGGR == PGH_MAX || AGGR == PGH_MIN);
+  constexpr float kPole = AGGR == PGH_MAX ? INFINITY : -INFINITY;
   const float4 ov = kExt ? outp[rest * v.c4 + ch] : make_float4(0.f, 0.f, 0.f, 0.f);
   float4 wgt = g;
   if (AGGR != PGH_SUM) {
@@ -277,7 +287,10 @@ masked_pool_bwd_warp_kernel(const float4* __restrict__ data, const unsigned char
           }
 #pragma unroll
         for (int u = 0; u < 8; ++u)
-          if (u < n) { c0 += x[u].x == ov.x; c1 += x[u].y == ov.y; c2 += x[u].z == ov.z; c3 += x[u].w == ov.w; }
+          if (u < n) {
+            c0 = pool_tie(c0, x[u].x, ov.x, kPole); c1 = pool_tie(c1, x[u].y, ov.y, kPole);
+            c2 = pool_tie(c2, x[u].z, ov.z, kPole); c3 = pool_tie(c3, x[u].w, ov.w, kPole);
+          }
       }
     }
     if (!kExt) c1 = c2 = c3 = c0;
@@ -291,7 +304,10 @@ masked_pool_bwd_warp_kernel(const float4* __restrict__ data, const unsigned char
       if (wid == 0) {
         int4 t = make_int4(0, 0, 0, 0);
 #pragma unroll
-        for (int q = 0; q < 8; ++q) { const int4 u = pc[q][lane]; t.x += u.x; t.y += u.y; t.z += u.z; t.w += u.w; }
+        for (int q = 0; q < 8; ++q) {
+          const int4 u = pc[q][lane];
+          t = make_int4(pool_cnt_add(t.x, u.x), pool_cnt_add(t.y, u.y), pool_cnt_add(t.z, u.z), pool_cnt_add(t.w, u.w));
+        }
         cpc[lane] = t;
       }
       cluster.sync();
@@ -299,12 +315,13 @@ masked_pool_bwd_warp_kernel(const float4* __restrict__ data, const unsigned char
 #pragma unroll
       for (int q = 0; q < kPoolCluster; ++q) {
         const int4 t = cluster.map_shared_rank(&cpc[0], q)[lane];
-        c0 += t.x; c1 += t.y; c2 += t.z; c3 += t.w;
+        c0 = pool_cnt_add(c0, t.x); c1 = pool_cnt_add(c1, t.y);
+        c2 = pool_cnt_add(c2, t.z); c3 = pool_cnt_add(c3, t.w);
       }
       cluster.sync();                              // peers may exit only after everyone has read
     }
-    wgt = make_float4(c0 ? g.x / (float)c0 : 0.f, c1 ? g.y / (float)c1 : 0.f,
-                      c2 ? g.z / (float)c2 : 0.f, c3 ? g.w / (float)c3 : 0.f);
+    wgt = make_float4(c0 > 0 ? g.x / (float)c0 : 0.f, c1 > 0 ? g.y / (float)c1 : 0.f,
+                      c2 > 0 ? g.z / (float)c2 : 0.f, c3 > 0 ? g.w / (float)c3 : 0.f);
   }
   const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
   for (int rc = sub * 32; rc < v.red; rc += kStep) {
@@ -354,23 +371,26 @@ __global__ void masked_pool_bwd_kernel(const float4* __restrict__ data,
   const long long pstep = v.inner, dstep = (long long)v.inner * v.c4;
   const float4 g = g_out[idx];
   constexpr bool kExt = (AGGR == PGH_MAX || AGGR == PGH_MIN);
+  constexpr float kPole = AGGR == PGH_MAX ? INFINITY : -INFINITY;
   const float4 ov = kExt ? outp[idx] : make_float4(0.f, 0.f, 0.f, 0.f);
   float4 w = g;
   if (AGGR != PGH_SUM) {
-    // mean: 1/#valid ; max/min: 1/#ties per channel (torch.amax backward splits evenly)
+    // mean: 1/#valid ; max/min: 1/#ties per channel (torch.amax backward splits evenly), none
+    // where a valid entry is the infinite extreme (pool_tie)
     int c0 = 0, c1 = 0, c2 = 0, c3 = 0;
     for (int r = 0; r < v.red; ++r) {
       if (!__ldg(mp + r * pstep)) continue;
       if (kExt) {
         const float4 x = __ldg(dp + r * dstep);
-        c0 += x.x == ov.x; c1 += x.y == ov.y; c2 += x.z == ov.z; c3 += x.w == ov.w;
+        c0 = pool_tie(c0, x.x, ov.x, kPole); c1 = pool_tie(c1, x.y, ov.y, kPole);
+        c2 = pool_tie(c2, x.z, ov.z, kPole); c3 = pool_tie(c3, x.w, ov.w, kPole);
       } else {
         ++c0;
       }
     }
     if (!kExt) c1 = c2 = c3 = c0;
-    w = make_float4(c0 ? g.x / (float)c0 : 0.f, c1 ? g.y / (float)c1 : 0.f,
-                    c2 ? g.z / (float)c2 : 0.f, c3 ? g.w / (float)c3 : 0.f);
+    w = make_float4(c0 > 0 ? g.x / (float)c0 : 0.f, c1 > 0 ? g.y / (float)c1 : 0.f,
+                    c2 > 0 ? g.z / (float)c2 : 0.f, c3 > 0 ? g.w / (float)c3 : 0.f);
   }
   for (int r = 0; r < v.red; ++r) {
     float4 val = make_float4(0.f, 0.f, 0.f, 0.f);

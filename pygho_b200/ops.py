@@ -833,14 +833,27 @@ def _ext3(eX: Optional[Tensor], tx: bool, eY: Optional[Tensor], ty: bool, eM: Op
     return ext, order
 
 
+def _tc_tile_bytes(n_i: int, n_j: int, n_k: int) -> int:
+    """Shared memory of the tensor-core kernels' tiles: 8 channel tiles of each operand with K
+    padded to 8, plus the mask tile (mamamm_tc_launch in csrc/mamamm_tc.cu; keep in step)."""
+    k_pad, n_pad = -(-n_j // 8) * 8, -(-n_k // 16) * 16
+    sbo = k_pad // 4 * 128
+    ts_a, ts_b = -(-n_i // 8) * sbo + 16, -(-n_k // 8) * sbo + 16
+    off_b = -(-8 * ts_a // 128) * 128
+    total = max(off_b + 8 * ts_b, 7 * ts_a + 16 * sbo, off_b + 7 * ts_b + n_pad // 8 * sbo)
+    return -(-total // 128) * 128 + -(-(n_i * n_k) // 128) * 128
+
+
 def mamamm_algo_for(algo: int, n_i: int, n_j: int, n_k: int, dense: int) -> int:
     """The tensor-core kernels (algo 1 / 2) hold one (n_i x n_j) and one (n_j x n_k) tile per
-    channel: n_i, n_j <= 128, n_k <= 64, dense % 8 == 0.  Anything else runs on the exact-fp32 kernel
-    (algo 0).  Decided per CALL: the gradient contractions of a forward that fits may
-    not fit themselves (their (n_i, n_j, n_k) roles are permuted).  algo 4 (exact fp32 from a
-    TMA-fed shared-memory ring, csrc/mamamm_smem.cu) takes any shape: the library itself runs the
-    shapes its ring cannot hold on algo 0."""
-    if algo in (1, 2) and (dense % 8 != 0 or n_i > 128 or n_k > 64 or n_j > 128):
+    channel: n_i, n_j <= 128, n_k <= 64, dense % 8 == 0, and the 8-channel tiles of both operands
+    within 227 KB of shared memory.  Anything else runs on the exact-fp32 kernel (algo 0).
+    Decided per CALL: the gradient contractions of a forward that fits may not fit themselves
+    (their (n_i, n_j, n_k) roles are permuted).  algo 4
+    (exact fp32 from a TMA-fed shared-memory ring, csrc/mamamm_smem.cu) takes any shape: the
+    library itself runs the shapes its ring cannot hold on algo 0."""
+    if algo in (1, 2) and (dense % 8 != 0 or n_i > 128 or n_k > 64 or n_j > 128
+                           or _tc_tile_bytes(n_i, n_j, n_k) > 227 * 1024):
         return 0
     return algo
 

@@ -204,7 +204,7 @@ def test_ppgn_dense_conv_matches_reference_golden(golden, monkeypatch, algo, tol
         close(p.grad, g[f"grad.{k}"], 1e-4 * tol)
 
 
-@pytest.mark.parametrize("algo,tol", [(0, 1.0), (2, 50.0)])
+@pytest.mark.parametrize("algo,tol", [(0, 1.0), (2, 50.0), (4, 1.0)])
 def test_ma_model_matches_oracle_model(monkeypatch, algo, tol):
     """Dense PPGN model (example/zinc.py:155-219; bench.py --workload ppgn_dd) on ragged graphs:
     prediction, loss and every parameter gradient against the CPU oracle model."""
