@@ -1,6 +1,8 @@
 """GPU tests of evaluation on the fused path: the eval epilogue of the Linear GEMM
-(ops.linear_bn_eval, csrc/linear_stats.cu), its dispatch from the tuplewise MLP, eval-mode
-model parity with the oracle models, and graph-replayed prediction (static.StaticPredictor)."""
+(ops.linear_bn_eval, csrc/linear_stats.cu) against float64 per element, with the bound and the
+GEMM reference of tests/test_gpu_linear_stats.py (its module docstring derives them), its dispatch
+from the tuplewise MLP, eval-mode model parity with the oracle models, and graph-replayed prediction
+(static.StaticPredictor)."""
 import contextlib
 import copy
 
@@ -9,10 +11,20 @@ import pytest
 import torch
 
 from oracle import model_oracle as MO
+from test_gpu_linear_stats import (EPS, EPS32, NAN, RATIOS, SAT, U, check_bound, gemm_bound, gemm_ref, gen,
+                                   same_bits, set_pdl, split_of)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
 ACTS = {"none": 0, "silu": 1, "relu": 2}
+
+
+@pytest.fixture(scope="module", autouse=True)
+def _report_ratios():
+    yield
+    worst = {k: v for k, v in RATIOS.items() if k.startswith("eval")}
+    if worst:
+        print("\nworst |error| / bound: " + ", ".join(f"{k} {v:.3g}" for k, v in sorted(worst.items())))
 
 
 def close(a, b, rtol):
@@ -82,39 +94,106 @@ def _reference(x, w, b, gamma, beta, rm, rv, eps, act, res):
     return z if res is None else z + d(res)
 
 
-FLAGS = [(True, True, True), (False, False, False), (True, False, True), (False, True, False)]
-CASES = [(M, K, N, act, f) for N in (128, 256, 384) for K in (128, 384) for M in (4096, 4097)
-         for act in ACTS for f in FLAGS]
-CASES += [(230147, 384, 128, "silu", (True, True, True)), (230147, 384, 384, "silu", (True, True, True))]
+def eval_operands(M, K, N, bias, affine, residual, seed):
+    g = gen(seed)
+    x = torch.randn(M, K, device=DEV, generator=g)
+    w = torch.randn(N, K, device=DEV, generator=g) / K ** 0.5
+    b = torch.randn(N, device=DEV, generator=g) if bias else None
+    gamma = (torch.rand(N, device=DEV, generator=g) + 0.5) * torch.where(
+        torch.rand(N, device=DEV, generator=g) < 0.3, -1.0, 1.0) if affine else None
+    beta = torch.randn(N, device=DEV, generator=g) if affine else None
+    rm = torch.randn(N, device=DEV, generator=g) * 0.5
+    rv = 10.0 ** (torch.rand(N, device=DEV, generator=g) * 4 - 2)        # 1e-2 .. 1e2
+    res = torch.randn(M, N, device=DEV, generator=g) if residual else None
+    return x, w, b, gamma, beta, rm, rv, res
 
 
-@pytest.mark.parametrize("M,K,N,act,flags", CASES)
-def test_linear_bn_eval_kernel_matches_fp64(M, K, N, act, flags):
-    """One pass of act((x W^T + b - rm) / sqrt(rv + eps) * gamma + beta) (+ r) against fp64 torch,
-    with non-trivial running statistics; TF32 tolerance as for linear_stats."""
+def silu_es(t):
+    """Relative error of s~ = 1 / (1 + __expf(-t)) (tests/test_gpu_batchnorm.py)."""
+    e = torch.exp(-t)
+    es = 2.0 * (3.0 + 1.173 * t.abs()) * U * e / (1.0 + e) + 3.0 * U
+    return torch.where(-t > SAT, torch.ones_like(es), es)
+
+
+def eval_reference(x, w, b, gamma, beta, rm, rv, act, res, n):
+    """float64 z over the first n rows and its bound (module docstring)."""
+    N, K = w.shape
+    y64, mag = gemm_ref(x, w, b, n)
+    d = lambda t, v: t.double() if t is not None else torch.full((N,), v, dtype=torch.float64, device=DEV)  # noqa: E731
+    g, be, bb = d(gamma, 1.0), d(beta, 0.0), d(b, 0.0)
+    s = g / torch.sqrt(rv.double() + EPS32)
+    es = 1.01 * 5.5 * U * s.abs()
+    shift = (bb - rm.double()) * s + be
+    eshift = (bb - rm.double()).abs() * es + U * (bb - rm.double()).abs() * s.abs() + U * shift.abs()
+    t = (y64 - bb) * s + shift
+    et = 1.01 * (s.abs() * gemm_bound(K, mag, y64, bias_term=False) + (y64 - bb).abs() * es + eshift
+                 + U * t.abs())
+    if act == "silu":
+        z = t * torch.sigmoid(t)
+        ez = 1.1 * et + 1.01 * z.abs() * silu_es(t)
+    else:
+        z, ez = (t.clamp(min=0.0) if act == "relu" else t), et
+    if res is not None:
+        z = z + res[:n].double()
+        ez = ez + 1.01 * U * (z.abs() + ez)
+    return z, ez
+
+
+def eval_three(op, args, what):
+    runs = [op(*args), op(*args)]
+    set_pdl(False)
+    try:
+        runs.append(op(*args))
+    finally:
+        set_pdl(True)
+    assert same_bits(runs[0], runs[1]) and same_bits(runs[0], runs[2]), what + ": launches differ"
+    return runs[0]
+
+
+def check_eval(M, K, N, act, flags, seed, n=None, pad=0.0):
     residual, bias, affine = flags
-    x, w, b, gamma, beta, rm, rv, res = _operands(M, K, N, bias, affine, residual, M + K + N)
+    x, w, b, gamma, beta, rm, rv, res = eval_operands(M, K, N, bias, affine, residual, seed)
+    n = M if n is None else n
+    rows_dev = None if n == M and not pad else torch.tensor([n], dtype=torch.int32, device=DEV)
+    if n < M:
+        x[n:] = pad
     rm0, rv0 = rm.clone(), rv.clone()
-    z = _kernel()(x, w, b, gamma, beta, rm, rv, 1e-5, ACTS[act], res, None)
-    want = _reference(x, w, b, gamma, beta, rm, rv, 1e-5, act, res)
-    assert z.shape == (M, N) and bool(torch.isfinite(z).all())
-    assert float((z.double() - want).abs().max()) <= 2e-3 * float(want.abs().max())
-    assert torch.equal(rm, rm0) and torch.equal(rv, rv0)
+    what = f"eval M={M} K={K} N={N} {act} {flags} n={n}"
+    z = eval_three(_kernel(), (x, w, b, gamma, beta, rm, rv, EPS, ACTS[act], res, rows_dev), what)
+    assert same_bits(rm, rm0) and same_bits(rv, rv0), what + ": running statistics changed"
+    assert z.shape == (M, N) and bool((z[n:].view(torch.int32) == 0).all()), what + ": pad rows not +0"
+    want, bound = eval_reference(x, w, b, gamma, beta, rm, rv, act, res, n)
+    check_bound("eval " + act, z[:n], want, bound, what)
+    return z, (x, w, b, gamma, beta, rm, rv, res)
 
 
-@pytest.mark.parametrize("N,residual", [(128, True), (384, False)])
+FLAGS = [(True, True, True), (False, False, False), (True, False, True), (False, True, False)]
+EVAL_CASES = [(M, K, N, act, f) for N in (128, 256, 384) for K in (128, 384) for M in (4096, 4097)
+              for act in ACTS for f in FLAGS]
+EVAL_CASES += [(230147, 384, 128, "silu", (True, True, True)), (230147, 384, 384, "silu", (True, True, True))]
+EVAL_CASES += [(M, K, N, act, (True, True, True)) for M, K in ((1, 32), (2049, 4096), (37889, 96))
+               for N in (128, 256, 384) for act in ("none", "silu")]
+
+
+@pytest.mark.parametrize("M,K,N,act,flags", EVAL_CASES)
+def test_linear_bn_eval_kernel_matches_fp64(M, K, N, act, flags):
+    """act((x W^T + b - rm) / sqrt(rv + eps) gamma + beta) (+ r) against float64 per element, with
+    running statistics far from (0, 1), gamma of both signs, and gamma / beta NULL; one CTA, one and
+    two groups, and CTAs with 3 and 13 tiles (the single accumulator buffer of N = 384 reused)."""
+    assert split_of(M)[:2] in {(1, 1), (17, 2), (32, 2), (33, 3), (148, 10)}
+    check_eval(M, K, N, act, flags, M + K + N)
+
+
+@pytest.mark.parametrize("N,residual", [(128, True), (256, False), (384, False), (384, True)])
 def test_linear_bn_eval_pad_rows(N, residual):
-    """rows_dev = n < M: rows >= n are exactly 0, rows < n equal the call on the first n rows bit
-    for bit."""
+    """rows_dev = n < M with NaN in the pad rows of x: rows >= n are exactly 0, rows < n are within
+    the bound and equal the call on the first n rows bit for bit."""
     M, K, n = 8192, 256, 5000
-    x, w, b, gamma, beta, rm, rv, res = _operands(M, K, N, True, True, residual, 7)
-    rows = torch.tensor([n], dtype=torch.int32, device=DEV)
-    op = _kernel()
-    z = op(x, w, b, gamma, beta, rm, rv, 1e-5, 1, res, rows)
-    z_n = op(x[:n].contiguous(), w, b, gamma, beta, rm, rv, 1e-5, 1,
-             None if res is None else res[:n].contiguous(), None)
-    assert float(z[n:].abs().max()) == 0.0
-    assert torch.equal(z[:n], z_n)
+    z, (x, w, b, gamma, beta, rm, rv, res) = check_eval(M, K, N, "silu", (residual, True, True), 7,
+                                                        n=n, pad=NAN)
+    z_n = _kernel()(x[:n].contiguous(), w, b, gamma, beta, rm, rv, EPS, 1,
+                             None if res is None else res[:n].contiguous(), None)
+    assert same_bits(z[:n], z_n)
 
 
 def _mlp(rows, cin, cout, act="silu", seed=0):
